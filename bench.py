@@ -1,7 +1,7 @@
 """Benchmark of the D3PM denoising-sampler hot path (BASELINE.json metric: codec tokens/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c4|c5]
-                    [--denoise-steps S] [--transition absorbing|uniform]
+                    [--denoise-steps S] [--transition absorbing|uniform] [--dump-outputs DIR]
 
 Workload (default c3 = BASELINE.json configs[2], the configuration the throughput metric is
 quoted on; it fits one GPU): full denoiser (d=1024, 12 layers, 16 heads, K=1024, 8 levels), 256
@@ -16,7 +16,9 @@ multi-GPU entry point, ``vall_e.b200.shard.generate_sharded`` around ``Diffusion
 `value` with the batch already resident in HBM, `e2e` from pinned host tensors with the gathered
 codes read back to the host.  Every utterance is synthesised from its GLOBAL id, and the Philox
 noise is keyed by it, so the generated codes — `codes_sha256` — do not depend on N.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  ``--dump-outputs DIR`` also writes the codes of the last timed step
+as ``DIR/codes.npy``, so two builds can be compared output for output; it applies to ``--impl ours``
+only (the CPU reference arm times single denoise steps of one utterance, not a batch's codes).
 """
 from __future__ import annotations
 
@@ -200,6 +202,17 @@ def run_reference(args, wl):
                         "seconds": c1_s, "value": 225 * 8 / c1_s, "unit": UNIT, "kind": c1.kind, "cores": c1.cores},
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, codes, resp_lens):
+    """What a caller of the timed path receives for the last timed batch, ``generate_sharded(..., packed=True)``:
+    the int16 codes (B, T_max, 8) in global utterance order and the frame counts, as float32 .npy (codes < 1024
+    are exact in float32).  The largest workload, c3, writes 256 x 750 x 8 codes: 6 MB."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "codes.npy", codes.numpy().astype(np.float32))
+    np.save(d / "resp_lens.npy", np.asarray(resp_lens, dtype=np.float32))
 
 
 def config_dict(wl, n_gpus):
@@ -456,6 +469,8 @@ def run_ours(args, wl):
                              "local_ms_min": min(rank_local_ms), "local_ms_max": max(rank_local_ms),
                              "note": "step = generate_sharded incl. the all-gather; local = this rank's reverse loop only"},
                 "gpu_launches": launches, "roofline": roofline, "latency": latency, "cpu_baseline": cpu_baseline}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, codes_dev_arm, resp_lens)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -474,7 +489,14 @@ def main():
                     help="override the workload's number of denoise steps (BASELINE configs[4] sweeps 10/25/50/100)")
     ap.add_argument("--transition", default=None, choices=["absorbing", "uniform"],
                     help="override the workload's transition (BASELINE configs[4] sweeps both)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the codes the last timed step generated to DIR/codes.npy (float32), with the frame "
+                         "counts in DIR/resp_lens.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.denoise_steps is not None or args.transition is not None:
         B, t_txt, t_prom, t_resp, timesteps, transition = WORKLOADS[args.workload]
         WORKLOADS[args.workload] = (B, t_txt, t_prom, t_resp,

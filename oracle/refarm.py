@@ -4,9 +4,8 @@ The reference's OWN modules as the CPU arm of ``bench.py`` (``--impl reference``
 ``cpu_baseline`` leg) and as a cross-check of the oracle port:
 
 * ``stage()`` — the committed recipe: copies ``vall_e/vall_e/{base,nar,ar_discrete}.py`` verbatim from
-  ``/root/reference`` into the git-ignored ``oracle/_ref/`` (it travels to the GPU box with the snapshot,
-  like the built ``.so``; it never enters the history).  Run by ``__graft_entry__.build()`` wherever the
-  reference checkout exists; a no-op elsewhere.
+  the reference checkout (``reference_root()``) into the git-ignored ``oracle/_ref/`` (it never enters the
+  history).  Run by ``__graft_entry__.build()``; a no-op where no checkout can be read.
 * ``load()`` — imports the staged files behind a shim package: the reference package itself cannot be
   imported (``vall_e/config.py:96`` needs omegaconf; ``ar_discrete.py:14,16`` import diffusers / timm, which
   are stubbed — only ``timm...Mlp`` is structurally needed and the benchmarked path never builds it).
@@ -24,6 +23,8 @@ The reference's OWN modules as the CPU arm of ``bench.py`` (``--impl reference``
 from __future__ import annotations
 
 import importlib.util
+import json
+import os
 import shutil
 import sys
 import types
@@ -32,17 +33,33 @@ from pathlib import Path
 import torch
 
 HERE = Path(__file__).resolve().parent
-REF_SRC = Path("/root/reference/vall_e/vall_e")
 STAGED = HERE / "_ref"
 FILES = ("base.py", "nar.py", "ar_discrete.py")
 
 
+def reference_root() -> Path | None:
+    """The reference checkout: ``VALL_E_REF`` (its repository root), else ``reference`` next to this repository,
+    else BASELINE.json's ``reference_path`` — the order of ``vall_e.emb``.  A location this user cannot read
+    counts as absent (os.path.isdir returns False where pathlib would raise PermissionError)."""
+    cands = [os.environ.get("VALL_E_REF"), str(HERE.parent.parent / "reference")]
+    try:
+        cands.append(json.loads((HERE.parent / "BASELINE.json").read_text()).get("reference_path"))
+    except (OSError, ValueError):
+        pass
+    for c in cands:
+        if c and os.path.isdir(os.path.join(c, "vall_e", "vall_e")):
+            return Path(c)
+    return None
+
+
 def stage() -> bool:
     """Copies the three reference modules into oracle/_ref/ (verbatim).  True if they are staged."""
-    if REF_SRC.is_dir():
+    root = reference_root()
+    src = root / "vall_e" / "vall_e" if root else None
+    if src is not None and all(os.path.isfile(src / f) for f in FILES):
         STAGED.mkdir(exist_ok=True)
         for f in FILES:
-            shutil.copyfile(REF_SRC / f, STAGED / f)
+            shutil.copyfile(src / f, STAGED / f)
     return available()
 
 
@@ -59,7 +76,8 @@ def load():
     if _mods is not None:
         return _mods
     if not available():
-        raise FileNotFoundError("oracle/_ref/ is not staged: run oracle.refarm.stage() where /root/reference exists")
+        raise FileNotFoundError("oracle/_ref/ is not staged: run oracle.refarm.stage() where a checkout of the "
+                                "reference can be read (see reference_root)")
     diffusers = types.ModuleType("diffusers")
     for n in ("UNet3DConditionModel", "UNet2DConditionModel", "DDPMScheduler",
               "CosineDPMSolverMultistepScheduler", "DDIMScheduler"):

@@ -53,7 +53,7 @@ def stub_audio_modules(monkeypatch, calls):
 
 
 def standin_reference_emb(root: Path):
-    """A stand-in checkout for boxes without /root/reference: the two functions of emb/qnt.py and the one of
+    """A stand-in checkout of the reference: the two functions of emb/qnt.py and the one of
     emb/g2p.py that ``python -m vall_e`` calls (__main__.py:56-58,72), over the same third-party APIs."""
     emb = root / "vall_e" / "emb"
     emb.mkdir(parents=True)

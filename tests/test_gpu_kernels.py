@@ -71,8 +71,9 @@ def test_gemm_plain(L, M, N, K, simt):
                                    (1027, 3072, 256)])     # the last: 144 tiles of 128x192 (16-bit outputs), one wave
 def test_gemm_epilogues(L, simt, M, N, K):
     A, W = _rand_bf16((M, K), 3), _rand_bf16((N, K), 4, K ** -0.5)
-    bias = torch.randn(N, device=DEV)
-    resid = torch.randn(M, N, device=DEV)
+    g = torch.Generator().manual_seed(5)
+    bias = torch.randn(N, generator=g).to(DEV)
+    resid = torch.randn(M, N, generator=g).to(DEV)
     acc = A.float() @ W.float().t()
     out = torch.empty(M, N, dtype=torch.float16, device=DEV)
     L.gemm_bf16(out, A, W, bias, epi=L.EPI_BIAS, simt=simt)
@@ -80,7 +81,10 @@ def test_gemm_epilogues(L, simt, M, N, K):
     out = torch.empty(M, N, dtype=torch.bfloat16, device=DEV)
     L.gemm_bf16(out, A, W, bias, epi=L.EPI_BIAS_GELU, simt=simt)
     ref = torch.nn.functional.gelu(acc + bias)
-    assert (out.float() - ref).abs().max().item() < 3e-2
+    # bf16 output: rounding alone is up to half an ulp, 2^-8 |ref| (0.031 at |ref| = 8); 1e-3 covers the fp32
+    # accumulation order and the GELU polynomial (< 4.5e-5)
+    err = (out.float() - ref).abs()
+    assert (err <= 1e-3 + 2.0 ** -8 * ref.abs()).all(), err.max().item()
     x = resid.clone()
     L.gemm_bf16(x, A, W, bias, residual=x, epi=L.EPI_BIAS_RESIDUAL, simt=simt)   # in place, as the model uses it
     assert (x - (resid + acc + bias)).abs().max().item() < 2e-3

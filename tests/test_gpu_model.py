@@ -582,12 +582,9 @@ def test_cli_main_end_to_end(tmp_path, monkeypatch):
     """``python -m vall_e <text> <ref.wav> <out.wav> --ar-ckpt <Diffusion pickle>`` in-process, all the way to
     the written file: prompt through the (stubbed) EnCodec wrapper of ``vall_e.emb.qnt``, phones through
     ``vall_e.emb.g2p``, the reverse loop on the CUDA kernels, the codes back through ``qnt.decode_to_file``.
-    ``vall_e.emb`` executes the reference's own files where a checkout exists, else a stand-in checkout."""
-    from pathlib import Path
+    ``vall_e.emb`` executes the files of a stand-in checkout of the reference, written by the test."""
     from cli_helpers import run_cli, standin_reference_emb
-    ref = Path("/root/reference")
-    if not (ref / "vall_e" / "emb" / "qnt.py").is_file():
-        ref = standin_reference_emb(tmp_path / "standin")
+    ref = standin_reference_emb(tmp_path / "standin")
     main, calls, out = run_cli(tmp_path, monkeypatch, "cuda", ref)
     main()
     assert out.exists()

@@ -90,13 +90,15 @@ def test_denoiser_diffusion_matches_reference(golden_dir):
 
 def test_reference_arm_runs_the_staged_reference_modules():
     """oracle/refarm.py (the CPU arm of bench.py): the reference's own modules from oracle/_ref — staged by
-    build() where the reference checkout exists — run one denoise step, and the oracle port reproduces their
-    logits on the same weights (fp32, <= 5e-5) and their posterior (bit-exact), live, not only through fixtures."""
+    build() wherever a reference checkout can be read (refarm.reference_root) — run one denoise step, and the
+    oracle port reproduces their logits on the same weights (fp32, <= 5e-5) and their posterior (bit-exact),
+    live, not only through fixtures."""
     from oracle import denoiser as on
     from oracle import refarm
     from oracle.d3pm import D3PM
     if not refarm.stage():
-        pytest.skip("oracle/_ref not staged (no reference checkout on this box)")
+        pytest.skip("oracle/_ref not staged: no readable reference checkout (VALL_E_REF, ../reference or "
+                    "BASELINE.json reference_path)")
     g = torch.Generator().manual_seed(3)
     text, proms = torch.randint(1, 1025, (7,), generator=g), torch.randint(0, 1025, (11, 8), generator=g)
     S = 6

@@ -1,8 +1,11 @@
 """Config base: frozen dataclass filled from ``yaml=path`` and ``key=value`` command-line words,
 same convention as the reference (``vall_e/utils/config.py:78-106``) without the omegaconf
-dependency (not installed in this image).  As there: words containing ``=`` and no ``--`` are
-config words and are removed from ``sys.argv`` so argparse never sees them; keys that are not
-dataclass fields raise (structured merge); ``yaml=`` sets ``cfg_name`` from the file's path.
+dependency.  As there: ``key=value`` words without ``--`` whose key
+is a dataclass field, ``yaml`` or ``help`` are config words and are removed from ``sys.argv`` so
+argparse never sees them; other words stay for the program's own parser (a host program such as
+pytest may carry ``-o name=value`` in its argv when it imports this package); keys of
+``from_words`` and of the YAML that are not dataclass fields raise (structured merge); ``yaml=``
+sets ``cfg_name`` from the file's path.
 """
 from __future__ import annotations
 
@@ -86,9 +89,10 @@ class Config:
     def dumps(self):
         return json.dumps(asdict(self), indent=2, default=str)
 
-    @staticmethod
-    def _is_cfg_argv(s: str) -> bool:
-        return "=" in s and "--" not in s
+    @classmethod
+    def _is_cfg_argv(cls, s: str) -> bool:
+        key = s.split("=", 1)[0]
+        return "=" in s and "--" not in s and (key in ("yaml", "help") or key in {f.name for f in dataclasses.fields(cls)})
 
     @classmethod
     def from_words(cls, words: list[str]):
