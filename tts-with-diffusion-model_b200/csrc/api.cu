@@ -197,6 +197,10 @@ extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_d
       vb200::set_error("head_posterior_sample: null pointer");
       return VB200_ERR_INVALID;
     }
+    if (reinterpret_cast<uintptr_t>(bias) & 15) {                // the epilogue reads bias as float4
+      vb200::set_error("head_posterior_sample: bias must be 16-byte aligned");
+      return VB200_ERR_INVALID;
+    }
     return vb200::head_sample_fused(x_out, head_in_bf16, W_bf16, bias, x_t, row_utt, t_utt, utt, table, n_rows, d,
                              n_levels, K, S, static_cast<int>(tr), static_cast<int>(noise), seed,
                              head_in_dtype == VB200_F16, static_cast<cudaStream_t>(stream));
@@ -216,6 +220,10 @@ extern "C" int vb200_head_ce_loss(float* loss, const void* head_in_bf16, vb200_d
   if (n_rows == 0) return VB200_OK;
   if (!(loss && head_in_bf16 && W_bf16 && bias && targets)) {
     vb200::set_error("head_ce_loss: null pointer");
+    return VB200_ERR_INVALID;
+  }
+  if (reinterpret_cast<uintptr_t>(bias) & 15) {                  // the epilogue reads bias as float4
+    vb200::set_error("head_ce_loss: bias must be 16-byte aligned");
     return VB200_ERR_INVALID;
   }
   if (n_rows < 0 || n_levels < 1 || d <= 0 || d % 8 != 0 || K < 256 || K % 256 != 0) {

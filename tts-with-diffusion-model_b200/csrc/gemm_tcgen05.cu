@@ -369,17 +369,19 @@ static int launch_gemm(void* out, vb200_dtype dt, const void* A, vb200_dtype a_d
   if (t_narrow < best) { ctas = 1; narrow = true; best = t_narrow; }
   if (t_n64 < best) { ctas = 1; narrow = false; narrow64 = true; best = t_n64; }
   if (t_n192 < best) { ctas = 1; narrow = false; narrow64 = false; n192 = true; best = t_n192; }
-  // VB200_GEMM_TILE=pair|wide|narrow|n64 forces a tiling (A/B measurements, tools/gemm_small_probe.py)
+  // VB200_GEMM_TILE=pair|wide|narrow|n64|n192 forces a tiling (A/B measurements, tools/gemm_small_probe.py, and
+  // the per-tiling tests); where the forced tiling cannot apply, the 128x256 one runs instead
   static int tile_forced = -1;
   if (tile_forced < 0) {
     const char* e = getenv("VB200_GEMM_TILE");
-    tile_forced = !e ? 0 : e[0] == 'p' ? 1 : e[0] == 'w' ? 2 : (e[0] == 'n' && e[1] == 'a') ? 3 : (e[0] == 'n' && e[1] == '6') ? 4 : 0;
+    tile_forced = !e ? 0 : e[0] == 'p' ? 1 : e[0] == 'w' ? 2 : (e[0] == 'n' && e[1] == 'a') ? 3
+                : (e[0] == 'n' && e[1] == '6') ? 4 : (e[0] == 'n' && e[1] == '1') ? 5 : 0;
   }
   if (tile_forced) {
     ctas = tile_forced == 1 ? 2 : 1;
     narrow = tile_forced == 3 && N > 128;
     narrow64 = tile_forced == 4 && sizeof(OutT) == 4 && N > 64;
-    n192 = false;
+    n192 = tile_forced == 5 && sizeof(OutT) == 2 && N % 192 == 0;
   }
   const int bn = n192 ? 192 : narrow64 ? 64 : (narrow ? 128 : BN);
   CUtensorMap ta, tb, tout;
@@ -449,6 +451,8 @@ extern "C" int vb200_gemm_bf16(void* out, vb200_dtype out_dtype, const void* A, 
   VB_REQUIRE(N % 8 == 0, "gemm: N=%d must be a multiple of 8 (16-byte vector stores)", N);
   VB_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "gemm: out must be 16-byte aligned");
   VB_REQUIRE(epi == VB200_EPI_NONE || bias, "gemm: epilogue %d needs bias", static_cast<int>(epi));
+  VB_REQUIRE(epi == VB200_EPI_NONE || (reinterpret_cast<uintptr_t>(bias) & 15) == 0,
+             "gemm: bias must be 16-byte aligned (the epilogue reads it as float4)");
   VB_REQUIRE(epi != VB200_EPI_BIAS_RESIDUAL || (residual && out_dtype == VB200_F32),
              "gemm: BIAS_RESIDUAL needs residual and fp32 output");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
