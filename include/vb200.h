@@ -201,13 +201,12 @@ int vb200_posterior_sample_from_logits(int32_t* x_out, float* post_out, const vo
 /* H1 + P in one call (SURVEY.md §8a rows H1 and P; reference base.py:355,440 followed by
  * ar_discrete.py:347-375,401-420): logits = head_in (n_rows, d) x W (n_levels*K, d)^T + bias (both bf16 or both fp16) and
  * the reverse step of vb200_posterior_sample_from_logits on them.
- * For K % 256 == 0 and noise != VB200_NOISE_UNIFORMS this is ONE kernel: the reverse step runs as
- * the GEMM's epilogue (streaming reservoir sampling over the column tiles of a level, see
- * csrc/head_sample_tcgen05.cu) and `logits` is not touched.  Otherwise (arbitrary K, supplied
- * uniforms, or VB200_FUSED_HEAD=0) the logits go through the caller's scratch `logits`
- * (n_rows, n_levels*K) of logits_dtype and the standalone kernel.  The Philox draws of the two forms
- * differ (both are exact samples of the same posterior); greedy codes agree up to the fp16
- * rounding of the unfused logits. */
+ * Where vb200_head_fused(d, K, noise) holds this is ONE kernel: the reverse step runs as the GEMM's
+ * epilogue (streaming reservoir sampling over the column tiles of a level, see
+ * csrc/head_sample_tcgen05.cu) and `logits` is not touched.  Otherwise the logits go through the
+ * caller's scratch `logits` (n_rows, n_levels*K) of logits_dtype and the standalone kernel.  The Philox
+ * draws of the two forms differ (both are exact samples of the same posterior); greedy codes agree up
+ * to the fp16 rounding of the unfused logits. */
 int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
                                 const void* head_in, vb200_dtype head_in_dtype, const void* W,
                                 const float* bias, int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
@@ -215,6 +214,10 @@ int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits
                                 const int32_t* utt, const float* table, int32_t S,
                                 vb200_transition tr, vb200_noise noise, const float* uniforms,
                                 uint64_t seed, vb200_stream_t stream);
+
+/* 1 when vb200_head_posterior_sample runs as one kernel for this configuration (K % 256 == 0,
+ * 256 <= K <= 4096, d % 8 == 0, noise != VB200_NOISE_UNIFORMS), else 0.  Host-only call. */
+int vb200_head_fused(int32_t d, int32_t K, vb200_noise noise);
 
 /* Training forward's loss (SURVEY.md §8f.3; reference ar_discrete.py:684-687 `F.cross_entropy` on the
  * classifier output): loss[r, l] = -log softmax(head_in[r] W_l^T + b_l)[targets[r, l]], float32

@@ -51,6 +51,16 @@ def test_library_exports_every_declared_symbol(built_lib):
     assert L.load().vb200_version() == 100
 
 
+def test_head_fused_predicate(built_lib):
+    """vb200_head_fused is a host-only call: which configurations head_posterior_sample runs as one kernel."""
+    from vall_e.b200 import lib as L
+    assert L.head_fused(1024, 1024, L.NOISE_PHILOX) and L.head_fused(128, 256, L.NOISE_GREEDY)
+    assert L.head_fused(8, 4096, L.NOISE_PHILOX)
+    assert not L.head_fused(1024, 1024, L.NOISE_UNIFORMS)
+    for d, K in ((1024, 1025), (1024, 128), (1024, 4352), (100, 1024)):
+        assert not L.head_fused(d, K, L.NOISE_GREEDY), (d, K)
+
+
 def test_library_contains_blackwell_instructions(built_lib):
     sass = subprocess.run(["cuobjdump", "-sass", str(built_lib)], capture_output=True, text=True).stdout
     for mnemonic in ("UTCHMMA", "LDTM", "UTMALDG"):

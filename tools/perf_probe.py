@@ -75,8 +75,7 @@ def small_kernels():
 
 
 def head():
-    """classifier + reverse step through vb200_head_posterior_sample (fused unless VB200_FUSED_HEAD=0)"""
-    import os
+    """classifier + reverse step: fused (vb200_head_posterior_sample) and as gemm_bf16 + posterior_sample_from_logits"""
     sys.path.insert(0, str(ROOT / "tts-with-diffusion-model_b200"))
     from vall_e.vall_e import d3pm
     S, K, d = 51, 1024, 1024
@@ -93,10 +92,16 @@ def head():
         utt[:, L.U_RESP0] = torch.arange(B, device=dev, dtype=torch.int32) * 750
         t_utt = torch.full((B,), 30, dtype=torch.int32, device=dev)
         o = torch.empty(rows, 8, dtype=torch.int32, device=dev)
-        ms = timeit(lambda: L.head_posterior_sample(o, scratch, head_in, W, bias, x_t, row_utt, t_utt, utt, tab, 8, K,
-                                                    L.ABSORBING, L.NOISE_PHILOX, seed=1), iters=10)
-        print(f"head+posterior[fused={os.environ.get('VB200_FUSED_HEAD', '1')}] rows={rows}: {ms:.3f} ms "
-              f"({2*rows*8*K*d/ms/1e9:.0f} TFLOP/s of GEMM work)", flush=True)
+        def unfused():
+            L.gemm_bf16(scratch, head_in, W, bias, None, L.EPI_BIAS)
+            L.posterior_sample_from_logits(o, None, scratch, 8 * K, x_t, row_utt, t_utt, utt, tab, rows, 8, K,
+                                           L.ABSORBING, L.NOISE_PHILOX, seed=1)
+        for form, fn in (("fused", lambda: L.head_posterior_sample(o, None, head_in, W, bias, x_t, row_utt, t_utt, utt,
+                                                                    tab, 8, K, L.ABSORBING, L.NOISE_PHILOX, seed=1)),
+                         ("gemm+posterior", unfused)):
+            ms = timeit(fn, iters=10)
+            print(f"head+posterior[{form}] rows={rows}: {ms:.3f} ms "
+                  f"({2*rows*8*K*d/ms/1e9:.0f} TFLOP/s of GEMM work)", flush=True)
 
 
 if __name__ == "__main__":

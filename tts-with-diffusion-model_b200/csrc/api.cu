@@ -187,12 +187,7 @@ extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_d
     return VB200_ERR_INVALID;
   }
   // fused form: the reverse step runs as the GEMM's epilogue and `logits` stays untouched
-  static int fused = -1;
-  if (fused < 0) {
-    const char* e = getenv("VB200_FUSED_HEAD");
-    fused = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (fused && n_rows > 0 && vb200::head_sample_supported(d, K, static_cast<int>(noise))) {
+  if (n_rows > 0 && vb200_head_fused(d, K, noise)) {
     if (!(x_out && head_in_bf16 && W_bf16 && bias && x_t && row_utt && t_utt && utt && table)) {
       vb200::set_error("head_posterior_sample: null pointer");
       return VB200_ERR_INVALID;

@@ -31,7 +31,6 @@ int cuda_fail(cudaError_t e, const char* what);
 int num_sms();
 
 // classifier GEMM with the reverse step as its epilogue (head_sample_tcgen05.cu)
-bool head_sample_supported(int d, int K, int noise);
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias, const int32_t* x_t,
                       const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt, const float* table,
                       int n_rows, int d, int n_levels, int K, int S, int tr, int noise, uint64_t seed,

@@ -1,7 +1,7 @@
 // D3PM forward noising (row Q) and closed-form reverse step (row P), SURVEY.md §8(a).
 // One warp per token, O(K) work, fp32 in registers; the reference's dense (K,K) fp16 matmuls
 // (ar_discrete.py:337-345,377-400) collapse to a handful of per-timestep scalars.
-#include "common.cuh"
+#include "posterior.cuh"
 
 namespace vb200 {
 
@@ -171,21 +171,14 @@ __device__ __forceinline__ void load8<__half>(const __half* p, float (&v)[8]) {
   }
 }
 
-struct PostConst {
-  float f1_self, f1_oth;      // Q_t[j, x_t] for j == x_t / j != x_t
-  float a_gen, c_gen;         // f2_j = p_j * a + (1 - p_j) * c for generic j
-  float a_m, c_m;             // ... for j == m (absorbing only; equals generic for uniform)
-  int x_t, m;
-  bool raw;                   // t == 0: posterior logits are the raw logits (ar_discrete.py:374,407)
-};
-
-__device__ __forceinline__ float post_logit(const PostConst& pc, float logit, float p, int j) {
-  if (pc.raw) return logit;
-  const float f1 = (j == pc.x_t) ? pc.f1_self : pc.f1_oth;
-  const bool is_m = (j == pc.m);
-  const float a = is_m ? pc.a_m : pc.a_gen, c = is_m ? pc.c_m : pc.c_gen;
+// log w_j; raw (t == 0): the posterior logits are the raw logits (ar_discrete.py:374,407)
+__device__ __forceinline__ float post_logit(const PostScalars& s, bool raw, float logit, float p, int j) {
+  if (raw) return logit;
+  const float f1 = (j == s.x_t) ? s.f1_self : s.f1_oth;
+  const bool is_m = (j == s.m);
+  const float a = is_m ? s.a_m : s.a_gen, c = is_m ? s.c_m : s.c_gen;
   const float f2 = fmaf(p, a - c, c);
-  return logf(f1 + kEps) + logf(f2 + kEps);
+  return logf(f1) + logf(f2 + kEps);
 }
 
 template <typename T, int NOISE>
@@ -206,25 +199,8 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
        tok += gridDim.x * warps_per_block) {
     const int row = tok / n_levels, level = tok - row * n_levels;
     const int b = row_utt[row];
-    const int t = min(max(t_utt[b], 0), S - 1);
-    const int t1 = t > 0 ? t - 1 : 0;
-    const float* one = table + static_cast<size_t>(t) * VB200_TAB_STRIDE;
-    const float* cum = table + static_cast<size_t>(t1) * VB200_TAB_STRIDE;
-    PostConst pc;
-    pc.x_t = x_t_all[tok];
-    pc.m = (transition == VB200_ABSORBING) ? K / 2 : -1;
-    pc.raw = (t == 0);
-    if (transition == VB200_ABSORBING) {
-      const bool at_m = pc.x_t == pc.m;
-      pc.f1_self = at_m ? one[VB200_TAB_ONE_BOTH] : one[VB200_TAB_ONE_KEEP];
-      pc.f1_oth = at_m ? one[VB200_TAB_ONE_ABSORB] : one[VB200_TAB_ONE_OFF];
-      pc.a_gen = cum[VB200_TAB_CUM_KEEP]; pc.c_gen = cum[VB200_TAB_CUM_OFF];
-      pc.a_m = cum[VB200_TAB_CUM_BOTH];   pc.c_m = cum[VB200_TAB_CUM_ABSORB];
-    } else {
-      pc.f1_self = one[VB200_TAB_ONE_KEEP]; pc.f1_oth = one[VB200_TAB_ONE_OFF];
-      pc.a_gen = pc.a_m = cum[VB200_TAB_CUM_KEEP];
-      pc.c_gen = pc.c_m = cum[VB200_TAB_CUM_OFF];
-    }
+    const int t = clamp_timestep(t_utt[b], S);
+    const bool raw = t == 0;   // raw logits and no noise (nonzero_mask, ar_discrete.py:412-419)
     const T* lrow = logits + static_cast<size_t>(row) * ld_logits + static_cast<size_t>(level) * K;
 
     // pass 1: row max; pass 2: sum exp (the row is 2-4 KB and stays in L1 between passes)
@@ -251,18 +227,13 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
     }
     sum = warp_sum(sum);
     const float inv = 1.0f / sum;
+    const PostScalars ps = post_scalars(table, t, x_t_all[tok], K, transition);
 
     // Philox key: (seed) ; counter: (j/4, frame*n_levels+level, global utterance id, t)
-    uint32_t gid = 0, frame = 0;
-    if (NOISE == VB200_NOISE_PHILOX) {
-      const int32_t* ur = utt + static_cast<size_t>(b) * VB200_U_STRIDE;
-      gid = static_cast<uint32_t>(ur[VB200_U_GID]);
-      frame = static_cast<uint32_t>(row - ur[VB200_U_RESP0]);
-    }
+    const TokenKey key = NOISE == VB200_NOISE_PHILOX ? token_key(utt, b, row, level, n_levels) : TokenKey{0, 0};
     const Philox ph{seed_lo, seed_hi};
     const float* urow = (NOISE == VB200_NOISE_UNIFORMS) ? uniforms + static_cast<size_t>(tok) * K : nullptr;
     float* prow = post_out ? post_out + static_cast<size_t>(tok) * K : nullptr;
-    const bool noisy = !pc.raw;   // nonzero_mask, ar_discrete.py:412-419
 
     Best best{-INFINITY, 0x7fffffff};
     if (vec) {
@@ -270,8 +241,8 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
         float v[8]; load8<T>(lrow + j0, v);
         float g[8];
         if (NOISE == VB200_NOISE_PHILOX) {
-          const uint4 r0 = ph(j0 >> 2, frame * n_levels + level, gid, t);
-          const uint4 r1 = ph((j0 >> 2) + 1, frame * n_levels + level, gid, t);
+          const uint4 r0 = ph(j0 >> 2, key.tok, key.gid, t);
+          const uint4 r1 = ph((j0 >> 2) + 1, key.tok, key.gid, t);
           const uint32_t rr[8] = {r0.x, r0.y, r0.z, r0.w, r1.x, r1.y, r1.z, r1.w};
 #pragma unroll
           for (int i = 0; i < 8; ++i) g[i] = gumbel_fast(u01(rr[i]));
@@ -282,23 +253,23 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const int j = j0 + i;
-          const float pl = post_logit(pc, v[i], __expf(v[i] - mx) * inv, j);
+          const float pl = post_logit(ps, raw, v[i], __expf(v[i] - mx) * inv, j);
           if (prow) prow[j] = pl;
-          const float sc = (NOISE != VB200_NOISE_GREEDY && noisy) ? pl + g[i] : pl;
+          const float sc = (NOISE != VB200_NOISE_GREEDY && !raw) ? pl + g[i] : pl;
           best_update(best, sc, j);
         }
       }
     } else {
       for (int j = lane; j < K; j += 32) {
         const float l = load_logit<T>(lrow, j);
-        const float pl = post_logit(pc, l, __expf(l - mx) * inv, j);
+        const float pl = post_logit(ps, raw, l, __expf(l - mx) * inv, j);
         if (prow) prow[j] = pl;
         float sc = pl;
-        if (NOISE == VB200_NOISE_PHILOX && noisy) {
-          const uint4 r = ph(j >> 2, frame * n_levels + level, gid, t);
+        if (NOISE == VB200_NOISE_PHILOX && !raw) {
+          const uint4 r = ph(j >> 2, key.tok, key.gid, t);
           const uint32_t rr[4] = {r.x, r.y, r.z, r.w};
           sc += gumbel_fast(u01(rr[j & 3]));
-        } else if (NOISE == VB200_NOISE_UNIFORMS && noisy) {
+        } else if (NOISE == VB200_NOISE_UNIFORMS && !raw) {
           sc += gumbel_exact(__ldg(urow + j));
         }
         best_update(best, sc, j);
@@ -361,17 +332,11 @@ __device__ __forceinline__ float cvt1(Raw1<__nv_bfloat16> r) { return __bfloat16
 // are read from HBM exactly once (16-byte loads), softmax statistics stay in registers, and the
 // token is drawn by inverse CDF from ONE Philox uniform — an exact categorical sample, equal in
 // distribution to the reference's Gumbel-max over K uniforms (ar_discrete.py:402-419) at 1/K of
-// the random numbers and no per-class logarithm.
-//
-// With e_j = exp(l_j - max), Z = sum e_j, p_j = e_j / Z the unnormalised posterior weight is
-//   w_j = (f1_j + eps) (f2_j + eps),  f2_j + eps = p_j (a_j - c_j) + c_j + eps.
-// Every class except x_t (and the absorbing class m) shares f1 / a / c, so
-//   sum_j w_j = coef * Z + K * cst  (+ non-negative corrections dx, dm for the special classes)
-// is closed form; the per-class weights are only walked when the draw lands in the generic part.
-// Greedy mode (argmax of the same weights) needs no logarithm either.
+// the random numbers and no per-class logarithm.  The total weight is closed form (posterior.cuh);
+// the per-class weights are only walked when the draw lands in the generic part.
 //
 // A warp walks its tokens in batches of 32.  Everything about a token that is not its logits —
-// timestep, x_t, the table-derived coefficients, the Philox draw — is produced LANE-PARALLEL at the
+// timestep, x_t, the table-derived scalars, the Philox draw — is produced LANE-PARALLEL at the
 // head of the batch (lane k prepares the batch's k-th token) and handed out with shuffles, so no
 // token waits on the utterance -> timestep -> table chain of dependent loads and the ten Philox
 // rounds cost 1/32 of a token each.  The logits of token k+1 (packed, unconverted) are in flight
@@ -387,15 +352,13 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
   pdl_launch_dependents();
   pdl_wait();                                   // everything below reads / writes activations
   constexpr int NR = KC * 8;                  // logits per lane
-  constexpr float kLog2e = 1.4426950408889634f;
   constexpr unsigned kFull = 0xffffffffu;
   const int warps_per_block = blockDim.x >> 5;
   const int lane = threadIdx.x & 31;
   const int n_tok = n_rows * n_levels;
   const int stride = gridDim.x * warps_per_block;
   const int w0 = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
-  const bool absorbing = transition == VB200_ABSORBING;
-  const int m_abs = absorbing ? K / 2 : -1;
+  const int m_abs = transition == VB200_ABSORBING ? K / 2 : -1;
   const int m_probe = K / 2;                  // column read for the absorbing class (unused otherwise)
 
   Raw8<T> nxt[KC];
@@ -413,54 +376,38 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
   for (int base = w0; base < n_tok; base += 32 * stride) {
     // ---- lane-parallel: everything but the logits of token `mine`
     const int mine = base + lane * stride;
-    int my_xt = 0, my_t = 0;
+    int my_t = 0;
     uint32_t my_rnd = 0;
-    float cA = 0.f, cC = 0.f, cF1s = 0.f, cDax = 0.f, cCx = 0.f, cAm = 0.f, cCm = 0.f;
+    PostScalars my{0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0, m_abs};
     if (mine < n_tok) {
       const int row = mine / n_levels, level = mine - row * n_levels;
       const int b = row_utt[row];
-      my_t = min(max(t_utt[b], 0), S - 1);
-      my_xt = x_t_all[mine];
-      const float* one = table + static_cast<size_t>(my_t) * VB200_TAB_STRIDE;
-      const float* cum = table + static_cast<size_t>(max(my_t - 1, 0)) * VB200_TAB_STRIDE;
-      const bool at_m = my_xt == m_abs;
-      const float f1_self = (absorbing && at_m ? one[VB200_TAB_ONE_BOTH] : one[VB200_TAB_ONE_KEEP]) + kEps;
-      const float f1_oth = (absorbing ? (at_m ? one[VB200_TAB_ONE_ABSORB] : one[VB200_TAB_ONE_OFF]) : one[VB200_TAB_ONE_OFF]) + kEps;
-      const float a_gen = cum[VB200_TAB_CUM_KEEP], c_gen = cum[VB200_TAB_CUM_OFF];
-      const float a_m = absorbing ? cum[VB200_TAB_CUM_BOTH] : a_gen, c_m = absorbing ? cum[VB200_TAB_CUM_ABSORB] : c_gen;
-      cA = (a_gen - c_gen) * f1_oth;              // generic class: w_j = cA / Z * e_j + cC
-      cC = (c_gen + kEps) * f1_oth;
-      cF1s = f1_self;                             // class x_t: w = cF1s * (e_x / Z * cDax + cCx)
-      cDax = at_m ? a_m - c_m : a_gen - c_gen;
-      cCx = (at_m ? c_m : c_gen) + kEps;
-      cAm = f1_oth * (a_m - c_m);                 // absorbing class (x_t != m): w = e_m / Z * cAm + cCm
-      cCm = f1_oth * (c_m + kEps);
+      my_t = clamp_timestep(t_utt[b], S);
+      my = post_scalars(table, my_t, x_t_all[mine], K, transition);
       if (NOISE == VB200_NOISE_PHILOX) {
-        const int32_t* ur = utt + static_cast<size_t>(b) * VB200_U_STRIDE;
-        const uint32_t gid = static_cast<uint32_t>(ur[VB200_U_GID]);
-        const uint32_t frame = static_cast<uint32_t>(row - ur[VB200_U_RESP0]);
+        const TokenKey key = token_key(utt, b, row, level, n_levels);
         const Philox ph{seed_lo, seed_hi};
-        my_rnd = ph(0xC0DEu, frame * n_levels + level, gid, my_t).x;
+        my_rnd = ph(0xC0DEu, key.tok, key.gid, my_t).x;
       }
     }
     // x_t of the next batch's first token, so that the last prefetch of this batch has its column
     const int nb = base + 32 * stride;
     const int nb_xt = nb < n_tok ? x_t_all[nb] : 0;
-    if (base == w0) prefetch(base, __shfl_sync(kFull, my_xt, 0));
+    if (base == w0) prefetch(base, __shfl_sync(kFull, my.x_t, 0));
 
 #pragma unroll 1
     for (int k = 0; k < 32; ++k) {
       const int tok = base + k * stride;
       if (tok >= n_tok) break;
       const int t = __shfl_sync(kFull, my_t, k);
-      const int x_t = __shfl_sync(kFull, my_xt, k);
+      const int x_t = __shfl_sync(kFull, my.x_t, k);
       // lane owns classes j = c*256 + lane*8 + i  (c < KC, i < 8) in registers v[c*8 + i]
       float v[NR];
 #pragma unroll
       for (int c = 0; c < KC; ++c) unpack8(nxt[c], v + c * 8);
       const float l_x = cvt1(nxt_lx), l_m = cvt1(nxt_lm);
       if (tok + stride < n_tok) {
-        const int xt_next = __shfl_sync(kFull, my_xt, (k + 1) & 31);
+        const int xt_next = __shfl_sync(kFull, my.x_t, (k + 1) & 31);
         prefetch(tok + stride, k == 31 ? nb_xt : xt_next);
       }
       // Row max; the arg max (lowest index wins ties) is only needed for greedy decoding and for
@@ -514,41 +461,31 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
         const float n = __shfl_up_sync(kFull, incl, o);
         if (lane >= o) incl += n;
       }
+      const float e_x = exp2f_fast(fmaf(l_x, kLog2e, mx_l2));
+      const float e_m = exp2f_fast(fmaf(l_m, kLog2e, mx_l2));
       const float Z = __shfl_sync(kFull, incl, 31);
       const float invZ = 1.0f / Z;
 
-      const bool at_m = x_t == m_abs;
-      const bool has_m = absorbing && !at_m;
-      const float coef = __shfl_sync(kFull, cA, k) * invZ;        // generic class: w_j = coef * e_j + cst
-      const float cst = __shfl_sync(kFull, cC, k);
-      // special classes: true weight minus what the generic formula assigns them (>= 0, see DESIGN.md)
-      const float e_x = exp2f_fast(fmaf(l_x, kLog2e, mx_l2));
-      const float w_x = __shfl_sync(kFull, cF1s, k) *
-                        fmaf(e_x * invZ, __shfl_sync(kFull, cDax, k), __shfl_sync(kFull, cCx, k));
-      const float dx = fmaxf(w_x - fmaf(e_x, coef, cst), 0.f);
-      const float e_m = exp2f_fast(fmaf(l_m, kLog2e, mx_l2));
-      const float w_m_all = fmaf(e_m * invZ, __shfl_sync(kFull, cAm, k), __shfl_sync(kFull, cCm, k));
-      const float w_m = has_m ? w_m_all : 0.f;
-      const float dm = has_m ? fmaxf(w_m_all - fmaf(e_m, coef, cst), 0.f) : 0.f;
+      // token k's scalars, from the lane that prepared them
+      const PostScalars ps{__shfl_sync(kFull, my.f1_self, k), __shfl_sync(kFull, my.f1_oth, k),
+                           __shfl_sync(kFull, my.a_gen, k),   __shfl_sync(kFull, my.c_gen, k),
+                           __shfl_sync(kFull, my.a_m, k),     __shfl_sync(kFull, my.c_m, k), x_t, m_abs};
+      const float coef = ps.cA() * invZ;                    // generic class: w_j = coef * e_j + cst
+      const float cst = ps.cst();
+      const PostSpecial w = post_special(ps, e_x, e_m, invZ, coef, cst);
       int pick;
       if (NOISE == VB200_NOISE_GREEDY) {
-        // generic weights are monotone in the logit, special classes only gain: compare three candidates
-        float best_w = fmaf(exp2f_fast(fmaf(top.v, kLog2e, mx_l2)), coef, cst);
-        pick = top.j;
-        if (top.j == x_t) best_w = w_x;
-        else if (top.j == m_abs) best_w = w_m;
-        if (w_x > best_w || (w_x == best_w && x_t < pick)) { best_w = w_x; pick = x_t; }
-        if (has_m && (w_m > best_w || (w_m == best_w && m_abs < pick))) { best_w = w_m; pick = m_abs; }
+        pick = post_greedy(ps, w, fmaf(exp2f_fast(fmaf(top.v, kLog2e, mx_l2)), coef, cst), top.j);
       } else {
         const uint32_t rnd = __shfl_sync(kFull, my_rnd, k);
         const float w_generic = fmaf(coef, Z, static_cast<float>(K) * cst);
-        float target = u01(rnd) * (w_generic + dx + dm);
-        if (target < dx) {
+        float target = u01(rnd) * (w_generic + w.dx + w.dm);
+        if (target < w.dx) {
           pick = x_t;
-        } else if (target < dx + dm) {
+        } else if (target < w.dx + w.dm) {
           pick = m_abs;
         } else {
-          target -= dx + dm;
+          target -= w.dx + w.dm;
           // lane-level CDF of the generic weights: lane sum = coef * sum(e) + NR * cst
           const float w_incl = fmaf(coef, incl, static_cast<float>((lane + 1) * NR) * cst);
           const unsigned ball = __ballot_sync(kFull, target < w_incl);

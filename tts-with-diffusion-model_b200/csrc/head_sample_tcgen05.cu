@@ -4,9 +4,8 @@
 // A token's posterior needs the softmax normaliser over all K classes of its level, i.e. over
 // K / 256 accumulator tiles, before anything can be drawn from it by inverse CDF — which is why the
 // unfused kernel (d3pm.cu) wants the finished logits.  The way around it is to decompose the
-// posterior instead of normalising it.  With e_j = exp(l_j - max), Z = sum e_j the unnormalised
-// weights are  w_j = coef e_j + cst  (+ corrections dx, dm >= 0 on the classes x_t and m), with
-// coef = cA / Z, so the total is  cA + K cst + dx + dm  and the draw is a MIXTURE:
+// posterior instead of normalising it: its total weight is  cA + K cst + dx + dm  (posterior.cuh),
+// so the draw is a MIXTURE:
 //     with probability  cA / total     a class from softmax(logits),
 //                       K cst / total  a uniform class,
 //                       dx / total     x_t,          dm / total   the absorbing class m.
@@ -23,7 +22,7 @@
 // consecutive column tiles, so that each epilogue thread (one accumulator row, half of the 256
 // columns of a tile) carries its token's streaming state in registers across the tiles of the
 // item; the two threads of a row merge at the end of the item and one of them writes the code.
-#include "common.cuh"
+#include "posterior.cuh"
 
 namespace vb200 {
 
@@ -39,7 +38,6 @@ constexpr int XCHG_WORDS = 12;                  // per row: what half 1 hands to
 constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_WARPS * 32 * ROW_BYTES + BM * XCHG_WORDS * 4 +
                            1024 /*align slack*/ + 256 /*barriers*/;
 constexpr uint32_t TMEM_COLS = 512;
-constexpr float kLog2e = 1.4426950408889634f;
 constexpr int MODE_CE = 100;                    // epilogue = cross-entropy against target classes (no sampling)
 }  // namespace hs
 
@@ -165,8 +163,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
     uint8_t* my_row = row_smem + (e * 32 + lane) * ROW_BYTES;
     const int sw = lane & 7;                   // 16-byte chunk index ^= row % 8: conflict-free 128-bit stores
     float* my_x = xchg + r_cta * XCHG_WORDS;
-    const bool absorbing = transition == VB200_ABSORBING;
-    const int m_abs = absorbing ? K / 2 : -1;
+    const int m_abs = transition == VB200_ABSORBING ? K / 2 : -1;
     const Philox ph{seed_lo, seed_hi};
     int it = 0;
     for (int item = item0; item < num_items; item += item_stride) {
@@ -181,10 +178,10 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
         x_t = x_t_all[static_cast<size_t>(grow) * n_levels + level];     // MODE_CE: the target class
         if (NOISE != MODE_CE) {
           b = row_utt[grow];
-          t = min(max(t_utt[b], 0), S - 1);
-          const int32_t* ur = utt + static_cast<size_t>(b) * VB200_U_STRIDE;
-          gid = static_cast<uint32_t>(ur[VB200_U_GID]);
-          key1 = static_cast<uint32_t>(grow - ur[VB200_U_RESP0]) * n_levels + level;
+          t = clamp_timestep(t_utt[b], S);
+          const TokenKey key = token_key(utt, b, grow, level, n_levels);
+          key1 = key.tok;
+          gid = key.gid;
         }
       }
       const bool need_arg = NOISE == VB200_NOISE_GREEDY || (NOISE != MODE_CE && t == 0);
@@ -330,34 +327,18 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
         } else if (t == 0) {
           pick = best_j;                                 // raw logits, no noise (ar_discrete.py:407,413)
         } else {
-          // per-timestep scalars (see posterior_fast_kernel in d3pm.cu for the derivation)
-          const float* one = table + static_cast<size_t>(t) * VB200_TAB_STRIDE;
-          const float* cum = table + static_cast<size_t>(t - 1) * VB200_TAB_STRIDE;
-          const bool at_m = x_t == m_abs;
-          const bool has_m = absorbing && !at_m;
-          const float f1_self = (absorbing && at_m ? one[VB200_TAB_ONE_BOTH] : one[VB200_TAB_ONE_KEEP]) + kEps;
-          const float f1_oth = (absorbing ? (at_m ? one[VB200_TAB_ONE_ABSORB] : one[VB200_TAB_ONE_OFF]) : one[VB200_TAB_ONE_OFF]) + kEps;
-          const float a_gen = cum[VB200_TAB_CUM_KEEP], c_gen = cum[VB200_TAB_CUM_OFF];
-          const float a_m = absorbing ? cum[VB200_TAB_CUM_BOTH] : a_gen, c_m = absorbing ? cum[VB200_TAB_CUM_ABSORB] : c_gen;
-          const float cA = (a_gen - c_gen) * f1_oth, cst = (c_gen + kEps) * f1_oth;
+          const PostScalars ps = post_scalars(table, t, x_t, K, transition);
+          const float cA = ps.cA(), cst = ps.cst();
           const float coef = cA * invZ;
-          const float w_x = f1_self * fmaf(e_x * invZ, at_m ? a_m - c_m : a_gen - c_gen, (at_m ? c_m : c_gen) + kEps);
-          const float dx = fmaxf(w_x - fmaf(e_x, coef, cst), 0.f);
-          const float w_m = has_m ? f1_oth * fmaf(e_m * invZ, a_m - c_m, c_m + kEps) : 0.f;
-          const float dm = has_m ? fmaxf(w_m - fmaf(e_m, coef, cst), 0.f) : 0.f;
+          const PostSpecial w = post_special(ps, e_x, e_m, invZ, coef, cst);
           if (NOISE == VB200_NOISE_GREEDY) {
-            float best_w = fmaf(exp2f_fast((best - m_f) * kLog2e), coef, cst);
-            pick = best_j;
-            if (best_j == x_t) best_w = w_x;
-            else if (best_j == m_abs) best_w = w_m;
-            if (w_x > best_w || (w_x == best_w && x_t < pick)) { best_w = w_x; pick = x_t; }
-            if (has_m && (w_m > best_w || (w_m == best_w && m_abs < pick))) { best_w = w_m; pick = m_abs; }
+            pick = post_greedy(ps, w, fmaf(exp2f_fast((best - m_f) * kLog2e), coef, cst), best_j);
           } else {
             const float w_uni = static_cast<float>(K) * cst;
-            const float target = u01(fin.y) * (cA + w_uni + dx + dm);
-            if (target < dx) pick = x_t;
-            else if (target < dx + dm) pick = m_abs;
-            else if (target < dx + dm + w_uni) pick = min(static_cast<int>(u01(fin.z) * K), K - 1);
+            const float target = u01(fin.y) * (cA + w_uni + w.dx + w.dm);
+            if (target < w.dx) pick = x_t;
+            else if (target < w.dx + w.dm) pick = m_abs;
+            else if (target < w.dx + w.dm + w_uni) pick = min(static_cast<int>(u01(fin.z) * K), K - 1);
             else pick = (u01(fin.w) * Z < Zb) ? cand_b : cand;     // softmax(logits): merge the two candidates
           }
         }
@@ -400,11 +381,6 @@ static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_
   return VB200_OK;
 }
 
-// true when the fused kernel covers this configuration (otherwise the caller runs GEMM + posterior kernel)
-bool head_sample_supported(int d, int K, int noise) {
-  return K % 256 == 0 && K >= 256 && K <= 4096 && d % 8 == 0 && noise != VB200_NOISE_UNIFORMS;
-}
-
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias,
                       const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt,
                       const float* table, int n_rows, int d, int n_levels, int K, int S, int tr, int noise,
@@ -425,3 +401,7 @@ int head_ce_fused(float* loss_out, const void* head_in, const void* W, const flo
 }
 
 }  // namespace vb200
+
+extern "C" int vb200_head_fused(int32_t d, int32_t K, vb200_noise noise) {
+  return K % 256 == 0 && K >= 256 && K <= 4096 && d % 8 == 0 && noise != VB200_NOISE_UNIFORMS;
+}

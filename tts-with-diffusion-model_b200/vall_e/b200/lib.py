@@ -50,6 +50,7 @@ PROTOTYPES = {
          _p],
         C.c_int),
     "vb200_q_sample_philox": ([_p] * 5 + [_i32, _i32, _i32, C.c_int, _u64, _p], C.c_int),
+    "vb200_head_fused": ([_i32, _i32, C.c_int], C.c_int),
     "vb200_head_ce_loss": ([_p, _p, C.c_int, _p, _p, _p, _i32, _i32, _i32, _i32, _p], C.c_int),
     "vb200_workspace_bytes": ([_i64, _i64, _i32, _i32, C.c_int, C.POINTER(C.c_int64)], C.c_int64),
     "vb200_step_timesteps": ([_p, _i32, _i32, _p], C.c_int),
@@ -236,10 +237,8 @@ def head_ce_loss(loss, head_in, W, bias, targets, n_levels, K):
 
 
 def head_fused(d, K, noise) -> bool:
-    """Mirrors head_sample_supported() in csrc/head_sample_tcgen05.cu: one kernel or two."""
-    import os
-    return (os.environ.get("VB200_FUSED_HEAD", "1")[:1] != "0" and K % 256 == 0 and 256 <= K <= 4096
-            and d % 8 == 0 and noise != NOISE_UNIFORMS)
+    """Whether head_posterior_sample runs as one kernel (else GEMM + standalone reverse step); host-only."""
+    return bool(load().vb200_head_fused(d, K, noise))
 
 
 WS_FIELDS = ("x", "h", "qkv", "att", "ff", "head_in", "logits")
