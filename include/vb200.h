@@ -139,16 +139,20 @@ int vb200_attn_varlen_simt(void* out_bf16, const void* qkv_bf16, const int32_t* 
                            vb200_stream_t stream);
 
 /* D3PM per-timestep scalar table, float32 (S, VB200_TAB_STRIDE), built on the host from the
- * fp16 transition tables (ar_discrete.py:257-277) — see vall_e/vall_e/d3pm.py. */
+ * fp16 transition tables (ar_discrete.py:257-277) — see vall_e/vall_e/d3pm.py.  The reverse step at t
+ * reads the ONE_* fields of row t and the CUM_* fields of row t-1.  A schedule table (d3pm.schedule_table,
+ * for a loop that jumps from t to s < t-1) holds Q_{t|s} = Q_{s+1}...Q_t in row t's ONE_* fields and
+ * Qbar_s in row t-1's CUM_* fields; it is for the reverse-step calls only, the q_sample calls take the
+ * plain table. */
 enum {
-  VB200_TAB_ONE_KEEP = 0,   /* Q_t[a,a]            (uniform: diagonal)           */
-  VB200_TAB_ONE_OFF = 1,    /* Q_t[a,b]            (uniform: off-diag; absorbing: 0) */
-  VB200_TAB_ONE_ABSORB = 2, /* Q_t[a,m]            (absorbing only)              */
-  VB200_TAB_ONE_BOTH = 3,   /* Q_t[m,m]            (absorbing only)              */
-  VB200_TAB_CUM_KEEP = 4,   /* Qbar_t[a,a]                                        */
-  VB200_TAB_CUM_OFF = 5,    /* Qbar_t[a,b]                                        */
-  VB200_TAB_CUM_ABSORB = 6, /* Qbar_t[a,m]                                        */
-  VB200_TAB_CUM_BOTH = 7,   /* Qbar_t[m,m]                                        */
+  VB200_TAB_ONE_KEEP = 0,   /* Q_t[a,a]   (uniform: diagonal)            schedule table, visited t: Q_{t|s}[a,a] */
+  VB200_TAB_ONE_OFF = 1,    /* Q_t[a,b]   (uniform: off-diag; absorbing: 0)                        Q_{t|s}[a,b] */
+  VB200_TAB_ONE_ABSORB = 2, /* Q_t[a,m]   (absorbing only)                                         Q_{t|s}[a,m] */
+  VB200_TAB_ONE_BOTH = 3,   /* Q_t[m,m]   (absorbing only)                                         Q_{t|s}[m,m] */
+  VB200_TAB_CUM_KEEP = 4,   /* Qbar_t[a,a]              schedule table, row t-1 of a t that jumps to s: Qbar_s[a,a] */
+  VB200_TAB_CUM_OFF = 5,    /* Qbar_t[a,b]                                                          Qbar_s[a,b] */
+  VB200_TAB_CUM_ABSORB = 6, /* Qbar_t[a,m]                                                          Qbar_s[a,m] */
+  VB200_TAB_CUM_BOTH = 7,   /* Qbar_t[m,m]                                                          Qbar_s[m,m] */
   VB200_TAB_LOG_KEEP = 8,   /* fp16 log(fp16(Qbar_t[a,a] + eps))   (q_sample logits)   */
   VB200_TAB_LOG_OFF = 9,
   VB200_TAB_LOG_ABSORB = 10,
@@ -247,6 +251,11 @@ int vb200_codes_to_bqt(int64_t* out, const int32_t* codes, const int32_t* utt, i
 
 /* reverse-loop helper (ar_discrete.py:750): t_utt[b] -= 1 for all b, on device (graph-capturable) */
 int vb200_step_timesteps(int32_t* t_utt, int32_t B, int32_t delta, vb200_stream_t stream);
+
+/* reverse-loop helper for a loop of fewer steps than timesteps: t_utt[b] = next_t[clamp(t_utt[b], 0, S-1)] for
+ * all b, on device (graph-capturable: one captured step replays for every step of a schedule).  next_t int32 (S) holds each
+ * visited timestep's successor (0 after the last).  Refuses null pointers and S < 1. */
+int vb200_step_timesteps_to(int32_t* t_utt, int32_t B, const int32_t* next_t, int32_t S, vb200_stream_t stream);
 
 #ifdef __cplusplus
 }

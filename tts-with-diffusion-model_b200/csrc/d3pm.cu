@@ -578,6 +578,14 @@ __global__ void step_timesteps_kernel(int32_t* t_utt, int B, int delta) {
   if (i < B) t_utt[i] += delta;
 }
 
+// t_utt[b] = next_t[t_utt[b]]: the successor of each utterance's timestep in the loop's schedule
+__global__ void step_timesteps_to_kernel(int32_t* t_utt, int B, const int32_t* __restrict__ next_t, int S) {
+  pdl_launch_dependents();
+  pdl_wait();                                   // everything below reads / writes activations
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < B) t_utt[i] = next_t[clamp_timestep(t_utt[i], S)];
+}
+
 }  // namespace vb200
 
 using namespace vb200;
@@ -670,6 +678,16 @@ extern "C" int vb200_step_timesteps(int32_t* t_utt, int32_t B, int32_t delta,
   if (B == 0) return VB200_OK;
   VB_CHECK_CUDA(launch_pdl(step_timesteps_kernel, dim3((B + 127) / 128), dim3(128), 0,
                            static_cast<cudaStream_t>(stream), 1, t_utt, B, delta));
+  VB_CHECK_CUDA(cudaGetLastError());
+  return VB200_OK;
+}
+
+extern "C" int vb200_step_timesteps_to(int32_t* t_utt, int32_t B, const int32_t* next_t, int32_t S,
+                                       vb200_stream_t stream) {
+  VB_REQUIRE(t_utt && next_t && B >= 0 && S >= 1, "step_timesteps_to: bad arguments");
+  if (B == 0) return VB200_OK;
+  VB_CHECK_CUDA(launch_pdl(step_timesteps_to_kernel, dim3((B + 127) / 128), dim3(128), 0,
+                           static_cast<cudaStream_t>(stream), 1, t_utt, B, next_t, S));
   VB_CHECK_CUDA(cudaGetLastError());
   return VB200_OK;
 }

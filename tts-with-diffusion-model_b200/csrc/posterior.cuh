@@ -30,7 +30,9 @@ struct PostScalars {
   __device__ __forceinline__ float cst() const { return (c_gen + kEps) * f1_oth; }
 };
 
-// t: clamped timestep.  The only reader of the Q_t / Qbar_{t-1} entries of the scalar table.
+// t: clamped timestep.  The only reader of the Q_t / Qbar_{t-1} entries of the scalar table.  A schedule table
+// (d3pm.schedule_table) holds Q_{t|s} and Qbar_s in those places for a step that jumps from t to s, so the same
+// reads give the jump posterior q(x_s | x_t, x̂0).
 __device__ __forceinline__ PostScalars post_scalars(const float* __restrict__ table, int t, int x_t, int K,
                                                     int transition) {
   const float* one = table + static_cast<size_t>(t) * VB200_TAB_STRIDE;

@@ -50,6 +50,8 @@ def main():
     parser.add_argument("--device", default="cuda")
     parser.add_argument("--frames", type=int, default=None, help="frames to generate (diffusion first stage)")
     parser.add_argument("--seed", type=int, default=0)
+    parser.add_argument("--steps", type=int, default=None,
+                        help="denoise steps of a diffusion first stage, 1 .. n_steps-1 (default: every timestep)")
     args = parser.parse_args()
 
     try:
@@ -66,7 +68,8 @@ def main():
 
     if isinstance(first, Diffusion):
         lens = [args.frames] if args.frames else None
-        resps_list = first.generate_audio(text_list=[phns], proms_list=[proms], resp_lens=lens, seed=args.seed)
+        resps_list = first.generate_audio(text_list=[phns], proms_list=[proms], resp_lens=lens, seed=args.seed,
+                                          sample_steps=args.steps)
     else:
         nar = _load(args.nar_ckpt, args.device)
         if isinstance(first, DiscreteAR):       # the reference's own D3PM class: level 0 by diffusion, 350 frames

@@ -299,12 +299,19 @@ class DenoiserEngine:
 
     def reverse_loop(self, lay: BatchLayout, ws: Workspace, x_t: torch.Tensor, table: torch.Tensor,
                      timesteps: int, transition: int, noise: int = L.NOISE_PHILOX, seed: int = 0,
-                     uniforms_fn=None, use_graph: bool = True, n_levels: int = 8, trace: list | None = None):
+                     uniforms_fn=None, use_graph: bool = True, n_levels: int = 8, trace: list | None = None,
+                     schedule=None, next_t: torch.Tensor | None = None):
         """One-shot form (tests): x_T -> x_0 in place on x_t int32 (M_resp, n_levels)."""
         ses = Session(self, lay, ws=ws, x_t=x_t)
         ses.run(table, timesteps, transition, noise=noise, seed=seed, uniforms_fn=uniforms_fn,
-                use_graph=use_graph, n_levels=n_levels, trace=trace)
+                use_graph=use_graph, n_levels=n_levels, trace=trace, schedule=schedule, next_t=next_t)
         return x_t
+
+
+def successor_tensor(timesteps: int, schedule, device) -> torch.Tensor:
+    """int32 (S,) next_t of ``schedule`` on ``device`` for ``vb200_step_timesteps_to``."""
+    from ..vall_e import d3pm
+    return torch.tensor(d3pm.successors(timesteps, schedule), dtype=torch.int32).to(device)
 
 
 class Session:
@@ -323,6 +330,7 @@ class Session:
         self.graph = None
         self.graph_key = None
         self.per_step_launches = 0
+        self._next_t = {}
 
     def signature(self):
         return (tuple(self.lay.t_txt), tuple(self.lay.t_prom), tuple(self.lay.t_resp))
@@ -350,18 +358,32 @@ class Session:
 
     def run(self, table: torch.Tensor, timesteps: int, transition: int, noise: int = L.NOISE_PHILOX,
             seed: int = 0, uniforms_fn=None, use_graph: bool = True, n_levels: int = 8,
-            trace: list | None = None) -> torch.Tensor:
-        """for t = S-1 .. 1 (never t = 0, as the reference, ar_discrete.py:750):
-        logits = denoiser(x_t, t); x_{t-1} = p_sample(logits, t, x_t), in place on self.x_t.
+            trace: list | None = None, schedule=None, next_t: torch.Tensor | None = None) -> torch.Tensor:
+        """for t in schedule (default S-1 .. 1; never t = 0, as the reference, ar_discrete.py:750):
+        logits = denoiser(x_t, t); x_{sigma(t)} = p_sample(logits, t, x_t), in place on self.x_t, where
+        sigma(t) is the next timestep of the schedule (0 after the last).  ``table`` must be the schedule's
+        (``d3pm.schedule_table``; ``d3pm.scalar_table`` for the default) and ``next_t`` its int32 (S,)
+        successor vector on the device (``successor_tensor``; built here when omitted).
         uniforms_fn(t) -> float32 (M_resp*n_levels, K) supplies the reference's torch.rand (parity)."""
+        from ..vall_e import d3pm
+        if schedule is None:
+            schedule = range(timesteps - 1, 0, -1)
+        schedule = d3pm.check_schedule(timesteps, schedule)
+        if next_t is None:
+            next_t = self._next_t.get(schedule)
+            if next_t is None:
+                next_t = self._next_t[schedule] = successor_tensor(timesteps, schedule, self.eng.w.device)
+        elif next_t.numel() != timesteps:
+            raise ValueError(f"next_t has {next_t.numel()} entries, the table {timesteps} timesteps")
         with torch.cuda.device(self.eng.w.device):
-            return self._run(table, timesteps, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace)
+            return self._run(table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels,
+                             trace)
 
-    def _run(self, table, timesteps, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace):
+    def _run(self, table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace):
         eng, lay, ws, x_t, t_utt = self.eng, self.lay, self.ws, self.x_t, self.t_utt
         w, dev = eng.w, eng.w.device
         K = w.n_out // n_levels
-        t_utt.fill_(timesteps - 1)
+        t_utt.fill_(schedule[0])
 
         def one_step(uniforms=None):
             if eng.profile is None and not eng.simt:
@@ -373,19 +395,19 @@ class Session:
                 logits = eng._forward(lay, ws, x_t, t_utt, True, None, True)
                 L.posterior_sample_from_logits(x_t, None, logits, w.n_out, x_t, lay.resp_row_utt, t_utt, lay.utt,
                                                table, lay.M_resp, n_levels, K, transition, noise, uniforms, seed)
-            L.step_timesteps(t_utt, -1)
+            L.step_timesteps_to(t_utt, next_t)
             eng.launches += 2
 
-        n_steps = timesteps - 1
+        n_steps = len(schedule)
         graph_ok = (use_graph and noise != L.NOISE_UNIFORMS and trace is None and n_steps > 2
                     and eng.profile is None)
         if not graph_ok:
-            for t in range(timesteps - 1, 0, -1):
+            for t in schedule:
                 one_step(uniforms_fn(t) if noise == L.NOISE_UNIFORMS else None)
                 if trace is not None:
                     trace.append(x_t.clone())
             return x_t
-        key = (table.data_ptr(), transition, noise, seed, n_levels)
+        key = (table.data_ptr(), next_t.data_ptr(), transition, noise, seed, n_levels)
         first = 0
         if self.graph is None or self.graph_key != key:
             # First step eagerly (also warms tensor-map caches and function attributes), then capture

@@ -54,6 +54,7 @@ PROTOTYPES = {
     "vb200_head_ce_loss": ([_p, _p, C.c_int, _p, _p, _p, _i32, _i32, _i32, _i32, _p], C.c_int),
     "vb200_workspace_bytes": ([_i64, _i64, _i32, _i32, C.c_int, C.POINTER(C.c_int64)], C.c_int64),
     "vb200_step_timesteps": ([_p, _i32, _i32, _p], C.c_int),
+    "vb200_step_timesteps_to": ([_p, _i32, _p, _i32, _p], C.c_int),
     "vb200_codes_to_bqt": ([_p, _p, _p, _i32, _i32, _i32, _i64, _p], C.c_int),
 }
 
@@ -255,3 +256,10 @@ def workspace_bytes(M, M_resp, d, n_out, logits_dtype):
 
 def step_timesteps(t_utt, delta):
     _check(load().vb200_step_timesteps(ptr(t_utt), t_utt.numel(), delta, stream()), "vb200_step_timesteps")
+
+
+def step_timesteps_to(t_utt, next_t):
+    """t_utt[b] = next_t[t_utt[b]] on device; next_t int32 (S,) (d3pm.successors)."""
+    _check(load().vb200_step_timesteps_to(ptr(t_utt), t_utt.numel(), ptr(next_t),
+                                          next_t.numel() if next_t is not None else 0, stream()),
+           "vb200_step_timesteps_to")

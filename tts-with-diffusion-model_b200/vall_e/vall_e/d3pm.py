@@ -52,7 +52,8 @@ def _onestep(beta_t: torch.Tensor, K: int, transition: str) -> torch.Tensor:
 
 @functools.lru_cache(maxsize=16)
 def scalar_table(timesteps: int, K: int, transition: str) -> torch.Tensor:
-    """float32 (S, TAB_STRIDE) table for vb200_q_sample / vb200_posterior_sample_from_logits."""
+    """float32 (S, TAB_STRIDE) table for vb200_q_sample / vb200_posterior_sample_from_logits (the reverse
+    step at every t = S-1 .. 1; ``schedule_table`` for fewer steps)."""
     betas = cosine_beta_schedule(timesteps + 1).to(torch.float16)     # ar_discrete.py:257
     m = K // 2
     a = 0 if m != 0 else 1
@@ -71,6 +72,73 @@ def scalar_table(timesteps: int, K: int, transition: str) -> torch.Tensor:
         # q_sample logits are formed in fp16: log(fp16(q) + eps) (ar_discrete.py:482)
         tab[t, L.TAB_LOG_KEEP:L.TAB_LOG_BOTH + 1] = torch.log(picks + EPS).float()
     return tab
+
+
+@functools.lru_cache(maxsize=64)
+def sample_schedule(timesteps: int, n: int) -> tuple[int, ...]:
+    """The ``n`` timesteps a reverse loop of ``n`` denoise steps visits: t_i = (S-1) - floor(i (S-1) / n),
+    i = 0 .. n-1, strictly decreasing from S-1; the step at t_i draws x_{t_{i+1}} (x_0 after the last).
+    ``n = S-1`` is the full loop S-1, ..., 1."""
+    S, n = int(timesteps), int(n)
+    if not 1 <= n <= S - 1:
+        raise ValueError(f"sample_steps must lie in [1, {S - 1}] for a model with {S} timesteps, got {n}")
+    return tuple((S - 1) - (i * (S - 1)) // n for i in range(n))
+
+
+def check_schedule(timesteps: int, schedule) -> tuple[int, ...]:
+    """``schedule`` as a tuple, or ValueError unless it is a non-empty, strictly decreasing list of
+    timesteps in [1, S-1]."""
+    sch = tuple(int(t) for t in schedule)
+    if not sch or not all(1 <= t <= timesteps - 1 for t in sch) or any(a <= b for a, b in zip(sch, sch[1:])):
+        raise ValueError(f"a schedule is a strictly decreasing list of timesteps in [1, {timesteps - 1}], got {sch}")
+    return sch
+
+
+def successors(timesteps: int, schedule) -> list[int]:
+    """next_t for ``vb200_step_timesteps_to``: next_t[t] = the timestep after t in ``schedule`` (0 after
+    the last), and t-1 (0 at t = 0) at every timestep the schedule does not visit."""
+    sch = check_schedule(timesteps, schedule)
+    nxt = [max(t - 1, 0) for t in range(timesteps)]
+    for t, s in zip(sch, sch[1:] + (0,)):
+        nxt[t] = s
+    return nxt
+
+
+@functools.lru_cache(maxsize=16)
+def _schedule_table(timesteps: int, K: int, transition: str, schedule: tuple) -> torch.Tensor:
+    plain = scalar_table(timesteps, K, transition)
+    tab = plain.clone()
+    betas = cosine_beta_schedule(timesteps + 1).to(torch.float16)
+    m = K // 2
+    a = 0 if m != 0 else 1
+    b = 1 if m != 1 else 2
+    for t, s in zip(schedule, schedule[1:] + (0,)):
+        if s == t - 1:
+            continue
+        jump = _onestep(betas[s + 1], K, transition)          # Q_{t|s} = Q_{s+1} ... Q_t, fp16 as scalar_table's Qbar
+        for u in range(s + 2, t + 1):
+            jump = torch.tensordot(jump, _onestep(betas[u], K, transition), dims=[[1], [0]])
+        tab[t, L.TAB_ONE_KEEP] = jump[a, a]
+        tab[t, L.TAB_ONE_OFF] = jump[a, b]
+        tab[t, L.TAB_ONE_ABSORB] = jump[a, m]
+        tab[t, L.TAB_ONE_BOTH] = jump[m, m]
+        tab[t - 1, L.TAB_CUM_KEEP:L.TAB_CUM_BOTH + 1] = plain[s, L.TAB_CUM_KEEP:L.TAB_CUM_BOTH + 1]
+    return tab
+
+
+def schedule_table(timesteps: int, K: int, transition: str, schedule) -> torch.Tensor:
+    """The scalar table of a reverse loop that visits ``schedule`` (``sample_schedule``, or any strictly
+    decreasing list in [1, S-1]), for the reverse-step kernels only.
+
+    The reverse step at t reads the Q entries of row t and the Qbar entries of row t-1 (``post_scalars``
+    in csrc/posterior.cuh).  For every visited t whose successor s = sigma(t) is not t-1, row t's ONE_*
+    fields hold Q_{t|s} = Q_{s+1} ... Q_t (the fp16 chain product, formed as ``scalar_table`` forms Qbar)
+    and row t-1's CUM_* fields hold Qbar_s, so the same closed form draws from the jump posterior
+    q(x_s | x_t, x̂0).  Every other entry is ``scalar_table``'s: for the full schedule the two tables are
+    equal.  A row's CUM_* fields no longer need to hold that row's own Qbar_t, so the table is for the
+    reverse step only: ``q_sample`` and the training forward keep getting ``scalar_table``.  This
+    function is the one place that knows that row layout.  Cached: do not modify the returned tensor."""
+    return _schedule_table(int(timesteps), int(K), transition, check_schedule(timesteps, schedule))
 
 
 @functools.lru_cache(maxsize=2)

@@ -12,12 +12,14 @@ Method names, argument order and tensor shapes follow the reference so parity te
 """
 from __future__ import annotations
 
+import numbers
+
 import torch
 import torch.nn.functional as F
 from torch import Tensor, nn
 
 from ..b200 import lib as L
-from ..b200.engine import BatchLayout, check_ids
+from ..b200.engine import BatchLayout, check_ids, successor_tensor
 from . import d3pm
 from .base import Base
 
@@ -44,6 +46,26 @@ class D3PMOps:
         key = (str(device), self.timesteps, self.num_classes, self.transition)
         if key not in cache:
             cache[key] = d3pm.scalar_table(self.timesteps, self.num_classes, self.transition).to(device)
+        return cache[key]
+
+    def _sample_steps(self, sample_steps) -> int:
+        """The number of denoise steps: ``sample_steps`` (None: S-1, every timestep), or ValueError for
+        anything but an integer in [1, S-1]."""
+        S = self.timesteps
+        n = S - 1 if sample_steps is None else sample_steps
+        if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n <= S - 1:
+            raise ValueError(f"sample_steps must be an integer in [1, {S - 1}] for a model with {S} timesteps, "
+                             f"got {sample_steps!r}")
+        return int(n)
+
+    def _sampling(self, device, n: int) -> tuple:
+        """(schedule, its table, its int32 (S,) successor vector) of a reverse loop of n denoise steps."""
+        cache = self.__dict__.setdefault("_tables", {})
+        key = ("schedule", str(device), self.timesteps, self.num_classes, self.transition, n)
+        if key not in cache:
+            sch = d3pm.sample_schedule(self.timesteps, n)
+            cache[key] = (sch, d3pm.schedule_table(self.timesteps, self.num_classes, self.transition, sch).to(device),
+                          successor_tensor(self.timesteps, sch, device))
         return cache[key]
 
     def _dense_log_qbar(self, device) -> Tensor:
@@ -182,11 +204,14 @@ class Diffusion(D3PMOps, Base):
     def generate_audio(self, text_list: list[Tensor], proms_list: list[Tensor], resps_list=None, *,
                        resp_lens: list[int] | None = None, seed: int = 0, greedy: bool = False,
                        uniforms_fn=None, gids=None, use_graph: bool = True, trace: list | None = None,
-                       to_host: bool = False, as_bqt: bool = False):
+                       to_host: bool = False, as_bqt: bool = False, sample_steps: int | None = None):
         """x_T -> x_0 for a batch of utterances; returns [LongTensor (t'', 8)].
 
         x_T is all ``mask_id`` for the absorbing transition (ar_discrete.py:699) and uniform random
-        codes for the uniform one; the loop runs t = S-1 .. 1 (ar_discrete.py:750).  ``resp_lens``
+        codes for the uniform one; the loop runs t = S-1 .. 1 (ar_discrete.py:750).  ``sample_steps``
+        = n in [1, S-1] runs n denoise steps instead, at t_i = (S-1) - floor(i (S-1) / n), each drawing
+        from the exact jump posterior q(x_{t_{i+1}} | x_{t_i}, x̂0) (``d3pm.schedule_table``); None is
+        S-1, the full loop.  ``resp_lens``
         gives the number of frames to generate per utterance (reference: fixed 350, :699);
         ``resps_list`` (optional) supplies x_T explicitly.  ``uniforms_fn(t)`` switches to the
         reference's noise convention (supplied U[0,1) of shape (sum t'' * 8, K)) for parity runs.
@@ -195,8 +220,10 @@ class Diffusion(D3PMOps, Base):
         ``emb/qnt.py:32-49 decode(codes (b q t))`` takes, zero-padded, so the EnCodec stage decodes
         the batch in one call instead of one ``t q -> 1 q t`` utterance at a time (SURVEY §8f.4).
         """
+        n_steps = self._sample_steps(sample_steps)
         eng = self.engine()
         dev = eng.w.device
+        schedule, table, next_t = self._sampling(dev, n_steps)
         if resps_list is not None:
             resp_lens = [len(r) for r in resps_list]
         elif resp_lens is None:
@@ -219,8 +246,9 @@ class Diffusion(D3PMOps, Base):
                 parts.append(torch.randint(0, self.num_classes, (n, self.n_levels), generator=g, dtype=torch.int32))
             x_t.copy_(torch.cat(parts), non_blocking=True)
         noise = L.NOISE_GREEDY if greedy else (L.NOISE_UNIFORMS if uniforms_fn is not None else L.NOISE_PHILOX)
-        ses.run(self._table(dev), self.timesteps, _TRANSITIONS[self.transition], noise=noise, seed=seed,
-                uniforms_fn=uniforms_fn, use_graph=use_graph, n_levels=self.n_levels, trace=trace)
+        ses.run(table, self.timesteps, _TRANSITIONS[self.transition], noise=noise, seed=seed,
+                uniforms_fn=uniforms_fn, use_graph=use_graph, n_levels=self.n_levels, trace=trace,
+                schedule=schedule, next_t=next_t)
         if as_bqt:        # one (B, 8, T_max) int64 tensor in the EnCodec decoder's layout + the frame counts
             bqt = torch.empty(lay.B, self.n_levels, max(lay.t_resp), dtype=torch.int64, device=dev)
             with torch.cuda.device(dev):
