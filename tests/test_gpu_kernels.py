@@ -7,6 +7,7 @@ import pytest
 import torch
 
 import error_bounds as eb
+import head_bounds as hb
 
 pytestmark = pytest.mark.gpu
 
@@ -489,8 +490,9 @@ def test_head_posterior_sample_fused_vs_separate_kernels(L):
 @pytest.mark.parametrize("act", [torch.bfloat16, torch.float16], ids=["bf16", "f16"])
 @pytest.mark.parametrize("rows,K,levels,d", [(77, 1024, 8, 128), (600, 512, 3, 64), (1000, 256, 1, 256)])
 def test_head_ce_loss_matches_torch(L, rows, K, levels, d, act):
-    """vb200_head_ce_loss (cross-entropy as the classifier GEMM's epilogue, no logits in memory)
-    against torch's cross-entropy on fp32 logits of the same 16-bit operands (both bf16 or both fp16)."""
+    """vb200_head_ce_loss (cross-entropy as the classifier GEMM's epilogue, no logits in memory) against the
+    float64 cross-entropy of the same 16-bit operands (both bf16 or both fp16), within the bound of
+    tests/head_bounds.py."""
     g = torch.Generator().manual_seed(rows)
     head_in = torch.randn(rows, d, generator=g).to(act).to(DEV)
     W = (torch.randn(levels * K, d, generator=g) * 0.4).bfloat16().to(act).to(DEV)
@@ -499,9 +501,9 @@ def test_head_ce_loss_matches_torch(L, rows, K, levels, d, act):
     tgt[0, 0], tgt[-1, -1] = 0, K - 1                    # first / last class of a level
     loss = torch.full((rows, levels), float("nan"), device=DEV)
     L.head_ce_loss(loss, head_in, W, bias, tgt, levels, K)
-    logits = (head_in.float() @ W.float().t() + bias).view(rows, levels, K)
-    ref = torch.nn.functional.cross_entropy(logits.reshape(-1, K), tgt.reshape(-1).long(), reduction="none")
-    assert (loss.view(-1) - ref).abs().max().item() < 2e-3
+    for lv, ref, bound in hb.level_references(head_in, W, bias, levels, K):
+        r, rest, unit = hb.ce_reference(ref, bound, tgt[:, lv])
+        eb.within(loss[:, lv], r, rest, unit, hb.C_CE, f"CE rows={rows} K={K} level {lv}")
 
 
 def test_q_sample_philox_uniform_transition_law(L):

@@ -149,32 +149,11 @@ def test_oracle_jump_posterior_equals_chained_one_step_posteriors(tr):
         assert checked >= K
 
 
-def _kernel_weights(tab, t, x_t, p, tr, eps):
-    """numpy restatement of post_scalars + post_special (csrc/posterior.cuh): the unnormalised weights the
-    reverse-step kernels give class j, reading row t's Q and row t-1's Qbar entries of ``tab``."""
-    from vall_e.b200 import lib as L
-    K = p.shape[-1]
-    one, cum = tab[t], tab[max(t - 1, 0)]
-    absorbing = tr == "absorbing"
-    m = K // 2 if absorbing else -1
-    at_m = m >= 0 and x_t == m
-    f1_self = (one[L.TAB_ONE_BOTH] if at_m else one[L.TAB_ONE_KEEP]) + eps
-    f1_oth = (one[L.TAB_ONE_ABSORB] if at_m else one[L.TAB_ONE_OFF]) + eps
-    a_gen, c_gen = cum[L.TAB_CUM_KEEP], cum[L.TAB_CUM_OFF]
-    a_m = cum[L.TAB_CUM_BOTH] if absorbing else a_gen
-    c_m = cum[L.TAB_CUM_ABSORB] if absorbing else c_gen
-    w = f1_oth * (p * (a_gen - c_gen) + c_gen + eps)
-    if m >= 0 and not at_m:
-        w[m] = f1_oth * (p[m] * (a_m - c_m) + c_m + eps)
-    a_x, c_x = (a_m, c_m) if at_m else (a_gen, c_gen)
-    w[x_t] = f1_self * (p[x_t] * (a_x - c_x) + c_x + eps)
-    return w
-
-
 @pytest.mark.parametrize("tr", ["absorbing", "uniform"])
 def test_schedule_table_gives_the_jump_posterior_through_the_kernel_reads(tr):
     """The row invariant, before any GPU run: what the kernels compute from a schedule table's rows t and
     t-1 is the oracle's jump posterior (within the reverse step's 2e-3 bar on log-probabilities)."""
+    from head_bounds import kernel_weights
     from jump_oracle import JumpD3PM, posterior_fp32
     from oracle.d3pm import EPS
     from vall_e.vall_e import d3pm as pd
@@ -182,18 +161,16 @@ def test_schedule_table_gives_the_jump_posterior_through_the_kernel_reads(tr):
     orc = JumpD3PM(S, K, tr)
     g = torch.Generator().manual_seed(7)
     for sch in ([S - 1], [S - 1, S // 2, S // 2 - 7, 3]):        # jumps S-1 -> 0, S-1 -> S/2, mid -> mid-7, 3 -> 0
-        tab = pd.schedule_table(S, K, tr, sch).double().numpy()
+        tab = pd.schedule_table(S, K, tr, sch).double()
         for t, s in zip(sch, sch[1:] + [0]):
             logits = (torch.randn(1, W, K, generator=g) * 3).to(torch.float16)
             x_t = torch.randint(0, K, (1, W), generator=g, dtype=torch.int32)
             x_t[0, ::2] = K // 2                                  # masked and unmasked x_t
             ref = torch.log_softmax(posterior_fp32(logits, x_t, torch.tensor([t]), orc, torch.tensor([s])).double(), -1)
-            p = torch.softmax(logits.double(), -1)[0].numpy()
-            for w_ in range(W):
-                lw = np.log(_kernel_weights(tab, t, int(x_t[0, w_]), p[w_], tr, EPS))
-                lw -= np.log(np.exp(lw - lw.max()).sum()) + lw.max()
-                err = np.abs(lw - ref[0, w_].numpy()).max()
-                assert err <= 2e-3, (tr, t, s, w_, err)
+            p = torch.softmax(logits.double(), -1)[0]
+            lw = torch.log_softmax(torch.log(kernel_weights(tab, torch.full((W,), t), x_t[0], p, tr, EPS)), -1)
+            err = (lw - ref[0]).abs().max(-1).values
+            assert float(err.max()) <= 2e-3, (tr, t, s, err.argmax().item(), float(err.max()))
 
 
 def test_sample_steps_out_of_range_raise_before_the_device_is_touched():
