@@ -202,6 +202,27 @@ int vb200_posterior_sample_from_logits(int32_t* x_out, float* post_out, const vo
                                        vb200_noise noise, const float* uniforms, uint64_t seed,
                                        vb200_stream_t stream);
 
+/* P with some x0 given (generate_audio(known_list=...): continuation, span editing, level-conditional
+ * sampling).  Same arguments as vb200_posterior_sample_from_logits plus `known`, int32 (n_rows, n_levels) or
+ * NULL (then exactly vb200_posterior_sample_from_logits).  known = -1: the token is drawn as there.  known = k
+ * in [0, K): the token's x0 is k and it draws from the ids form of q_posterior_logits (ar_discrete.py:347-375
+ * with x_start_logits=False),
+ *   x_s ~ q(x_s | x_t, x0 = k)  ∝  (Q_{t|s}[j, x_t] + eps) (Qbar_s[k, j] + eps),
+ * from the same table entries, eps and fp16 chain products as every other token (s = t-1 with the plain
+ * table).  Its logit row is not read: it may hold anything.  Philox and greedy draws are O(1) per token (at
+ * most three classes, {x_t, k, m}, weigh something of their own; greedy = the arg max, lowest class wins ties);
+ * with supplied uniforms the code is the Gumbel-arg max of the K posterior logits, and post_out receives those
+ * logits (0 at t == 0, where the reference returns its x_start_logits argument).  At t == 0 the code is k.
+ * Philox draws are keyed by (seed, frame * n_levels + level, global utterance id, t) like every other draw. */
+int vb200_posterior_sample_from_logits_known(int32_t* x_out, float* post_out, const void* logits,
+                                             vb200_dtype logits_dtype, int64_t ld_logits,
+                                             const int32_t* x_t, const int32_t* row_utt,
+                                             const int32_t* t_utt, const int32_t* utt,
+                                             const float* table, int32_t n_rows, int32_t n_levels,
+                                             int32_t K, int32_t S, vb200_transition tr,
+                                             vb200_noise noise, const float* uniforms, uint64_t seed,
+                                             const int32_t* known, vb200_stream_t stream);
+
 /* H1 + P in one call (SURVEY.md §8a rows H1 and P; reference base.py:355,440 followed by
  * ar_discrete.py:347-375,401-420): logits = head_in (n_rows, d) x W (n_levels*K, d)^T + bias (both bf16 or both fp16) and
  * the reverse step of vb200_posterior_sample_from_logits on them.
@@ -218,6 +239,20 @@ int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits
                                 const int32_t* utt, const float* table, int32_t S,
                                 vb200_transition tr, vb200_noise noise, const float* uniforms,
                                 uint64_t seed, vb200_stream_t stream);
+
+/* vb200_head_posterior_sample with some x0 given: `known` int32 (n_rows, n_levels) or NULL, with the semantics of
+ * vb200_posterior_sample_from_logits_known.  Same fused / unfused dispatch; in the fused kernel the classifier
+ * GEMM still runs in full and the epilogue takes the O(1) draw for a known token when the two halves of its row
+ * merge.  The returned codes are the step's draws: a caller that wants the given codes back overwrites the known
+ * positions once after its last step (Qbar_0 = Q_0 is not the identity and eps leaks mass, so the last draw can
+ * differ from k). */
+int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                      const void* head_in, vb200_dtype head_in_dtype, const void* W,
+                                      const float* bias, int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                      const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                      const int32_t* utt, const float* table, int32_t S,
+                                      vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                      uint64_t seed, const int32_t* known, vb200_stream_t stream);
 
 /* 1 when vb200_head_posterior_sample runs as one kernel for this configuration (K % 256 == 0,
  * 256 <= K <= 4096, d % 8 == 0, noise != VB200_NOISE_UNIFORMS), else 0.  Host-only call. */

@@ -174,14 +174,14 @@ extern "C" int64_t vb200_workspace_bytes(int64_t M, int64_t M_resp, int32_t d, i
   return total;
 }
 
-extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
-                                           const void* head_in_bf16, vb200_dtype head_in_dtype,
-                                           const void* W_bf16, const float* bias,
-                                           int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
-                                           const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
-                                           const int32_t* utt, const float* table, int32_t S,
-                                           vb200_transition tr, vb200_noise noise, const float* uniforms,
-                                           uint64_t seed, vb200_stream_t stream) {
+extern "C" int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                                 const void* head_in_bf16, vb200_dtype head_in_dtype,
+                                                 const void* W_bf16, const float* bias,
+                                                 int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                                 const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                                 const int32_t* utt, const float* table, int32_t S,
+                                                 vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                                 uint64_t seed, const int32_t* known, vb200_stream_t stream) {
   if (head_in_dtype != VB200_BF16 && head_in_dtype != VB200_F16) {
     vb200::set_error("head_posterior_sample: head_in must be bf16 or f16");
     return VB200_ERR_INVALID;
@@ -198,14 +198,28 @@ extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_d
     }
     return vb200::head_sample_fused(x_out, head_in_bf16, W_bf16, bias, x_t, row_utt, t_utt, utt, table, n_rows, d,
                              n_levels, K, S, static_cast<int>(tr), static_cast<int>(noise), seed,
-                             head_in_dtype == VB200_F16, static_cast<cudaStream_t>(stream));
+                             head_in_dtype == VB200_F16, known, static_cast<cudaStream_t>(stream));
   }
   const int rc = vb200_gemm_bf16(logits, logits_dtype, head_in_bf16, head_in_dtype, W_bf16, bias, nullptr, n_rows,
                                  n_levels * K, d, VB200_EPI_BIAS, stream);
   if (rc != VB200_OK) return rc;
-  return vb200_posterior_sample_from_logits(x_out, nullptr, logits, logits_dtype,
-                                            static_cast<int64_t>(n_levels) * K, x_t, row_utt, t_utt, utt,
-                                            table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, stream);
+  return vb200_posterior_sample_from_logits_known(x_out, nullptr, logits, logits_dtype,
+                                                  static_cast<int64_t>(n_levels) * K, x_t, row_utt, t_utt, utt,
+                                                  table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known,
+                                                  stream);
+}
+
+extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                           const void* head_in_bf16, vb200_dtype head_in_dtype,
+                                           const void* W_bf16, const float* bias,
+                                           int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                           const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                           const int32_t* utt, const float* table, int32_t S,
+                                           vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                           uint64_t seed, vb200_stream_t stream) {
+  return vb200_head_posterior_sample_known(x_out, logits, logits_dtype, head_in_bf16, head_in_dtype, W_bf16, bias,
+                                           n_rows, d, n_levels, K, x_t, row_utt, t_utt, utt, table, S, tr, noise,
+                                           uniforms, seed, nullptr, stream);
 }
 
 extern "C" int vb200_head_ce_loss(float* loss, const void* head_in_bf16, vb200_dtype head_in_dtype,

@@ -34,7 +34,7 @@ int num_sms();
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias, const int32_t* x_t,
                       const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt, const float* table,
                       int n_rows, int d, int n_levels, int K, int S, int tr, int noise, uint64_t seed,
-                      int in_f16, cudaStream_t st);
+                      int in_f16, const int32_t* known, cudaStream_t st);
 int head_ce_fused(float* loss_out, const void* head_in, const void* W, const float* bias, const int32_t* targets,
                   int n_rows, int d, int n_levels, int K, int in_f16, cudaStream_t st);
 

@@ -181,13 +181,50 @@ __device__ __forceinline__ float post_logit(const PostScalars& s, bool raw, floa
   return logf(f1) + logf(f2 + kEps);
 }
 
+// One warp's reverse step of a token whose x0 = k is given.  With supplied uniforms the code is the Gumbel-arg max
+// of its K posterior logits (the reference's noise convention); Philox and greedy take the O(1) form of
+// posterior.cuh, with the Philox counter posterior_fast_kernel uses, so the two kernels draw the same code.
+// post_out gets the logits of the ids form of q_posterior_logits (0 at t == 0, as the reference's
+// torch.where(t == 0, x_start_logits=False, ...) gives).
+template <int NOISE>
+__device__ __forceinline__ void known_token(int32_t* __restrict__ x_out, float* __restrict__ post_out,
+                                            const float* __restrict__ uniforms, const float* __restrict__ table,
+                                            const int32_t* __restrict__ utt, int tok, int b, int row, int level,
+                                            int n_levels, int t, int x_t, int k, int K, int transition,
+                                            uint32_t seed_lo, uint32_t seed_hi, int lane) {
+  const PostScalars ps = post_scalars(table, t, x_t, K, transition);
+  const bool raw = t == 0;
+  if (post_out || NOISE == VB200_NOISE_UNIFORMS) {
+    float* prow = post_out ? post_out + static_cast<size_t>(tok) * K : nullptr;
+    const float* urow = NOISE == VB200_NOISE_UNIFORMS ? uniforms + static_cast<size_t>(tok) * K : nullptr;
+    Best best{-INFINITY, 0x7fffffff};
+    for (int j = lane; j < K; j += 32) {
+      const float pl = raw ? 0.f : known_logit(ps, k, j);
+      if (prow) prow[j] = pl;
+      best_update(best, (NOISE == VB200_NOISE_UNIFORMS && !raw) ? pl + gumbel_exact(__ldg(urow + j)) : pl, j);
+    }
+    best = warp_best(best);
+    if (NOISE == VB200_NOISE_UNIFORMS && !raw) {
+      if (lane == 0) x_out[tok] = best.j;
+      return;
+    }
+  }
+  uint4 r = make_uint4(0, 0, 0, 0);
+  if (NOISE == VB200_NOISE_PHILOX) {
+    const TokenKey key = token_key(utt, b, row, level, n_levels);
+    r = Philox{seed_lo, seed_hi}(0xC0DEu, key.tok, key.gid, t);
+  }
+  const int pick = known_pick(ps, k, t, K, NOISE == VB200_NOISE_GREEDY, u01(r.x), u01(r.y));
+  if (lane == 0) x_out[tok] = pick;
+}
+
 template <typename T, int NOISE>
 __global__ void __launch_bounds__(256) posterior_sample_kernel(
     int32_t* __restrict__ x_out, float* __restrict__ post_out, const T* __restrict__ logits,
     int64_t ld_logits, const int32_t* __restrict__ x_t_all, const int32_t* __restrict__ row_utt,
     const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int K, int S, int transition,
-    const float* __restrict__ uniforms, uint32_t seed_lo, uint32_t seed_hi) {
+    const float* __restrict__ uniforms, uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known) {
   pdl_launch_dependents();
   pdl_wait();                                   // everything below reads / writes activations
   const int warps_per_block = blockDim.x >> 5;
@@ -201,6 +238,12 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
     const int b = row_utt[row];
     const int t = clamp_timestep(t_utt[b], S);
     const bool raw = t == 0;   // raw logits and no noise (nonzero_mask, ar_discrete.py:412-419)
+    const int kn = known ? known[tok] : -1;
+    if (kn >= 0) {             // x0 given: its law never reads the logits (posterior.cuh, known_pick)
+      known_token<NOISE>(x_out, post_out, uniforms, table, utt, tok, b, row, level, n_levels, t, x_t_all[tok], kn, K,
+                         transition, seed_lo, seed_hi, lane);
+      continue;
+    }
     const T* lrow = logits + static_cast<size_t>(row) * ld_logits + static_cast<size_t>(level) * K;
 
     // pass 1: row max; pass 2: sum exp (the row is 2-4 KB and stays in L1 between passes)
@@ -341,13 +384,15 @@ __device__ __forceinline__ float cvt1(Raw1<__nv_bfloat16> r) { return __bfloat16
 // token waits on the utterance -> timestep -> table chain of dependent loads and the ten Philox
 // rounds cost 1/32 of a token each.  The logits of token k+1 (packed, unconverted) are in flight
 // while token k is reduced.
-template <typename T, int KC, int NOISE>
+// KNOWN: `known` (x0 given for some tokens) is read; a template flag, so that without it the kernel is the
+// register-tight loop it was (a runtime branch costs spills at KC = 4).
+template <typename T, int KC, int NOISE, bool KNOWN>
 __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
     int32_t* __restrict__ x_out, const T* __restrict__ logits, int64_t ld_logits,
     const int32_t* __restrict__ x_t_all, const int32_t* __restrict__ row_utt,
     const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int S, int transition,
-    uint32_t seed_lo, uint32_t seed_hi) {
+    uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known) {
   constexpr int K = KC * 256;
   pdl_launch_dependents();
   pdl_wait();                                   // everything below reads / writes activations
@@ -378,16 +423,23 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
     const int mine = base + lane * stride;
     int my_t = 0;
     uint32_t my_rnd = 0;
+    int my_known = -1;                        // the code of a token whose x0 is given, drawn here in O(1)
     PostScalars my{0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0, m_abs};
     if (mine < n_tok) {
       const int row = mine / n_levels, level = mine - row * n_levels;
       const int b = row_utt[row];
       my_t = clamp_timestep(t_utt[b], S);
       my = post_scalars(table, my_t, x_t_all[mine], K, transition);
+      uint4 r = make_uint4(0, 0, 0, 0);
       if (NOISE == VB200_NOISE_PHILOX) {
         const TokenKey key = token_key(utt, b, row, level, n_levels);
         const Philox ph{seed_lo, seed_hi};
-        my_rnd = ph(0xC0DEu, key.tok, key.gid, my_t).x;
+        r = ph(0xC0DEu, key.tok, key.gid, my_t);
+        my_rnd = r.x;
+      }
+      if (KNOWN) {
+        const int kn = known[mine];
+        if (kn >= 0) my_known = known_pick(my, kn, my_t, K, NOISE == VB200_NOISE_GREEDY, u01(r.x), u01(r.y));
       }
     }
     // x_t of the next batch's first token, so that the last prefetch of this batch has its column
@@ -409,6 +461,13 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
       if (tok + stride < n_tok) {
         const int xt_next = __shfl_sync(kFull, my.x_t, (k + 1) & 31);
         prefetch(tok + stride, k == 31 ? nb_xt : xt_next);
+      }
+      if (KNOWN) {
+        const int kp = __shfl_sync(kFull, my_known, k);
+        if (kp >= 0) {
+          if (lane == 0) x_out[tok] = kp;
+          continue;
+        }
       }
       // Row max; the arg max (lowest index wins ties) is only needed for greedy decoding and for
       // t == 0 (raw logits, no noise, ar_discrete.py:407,413), so the sampling path pays for a plain max.
@@ -529,7 +588,7 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
                             const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
                             const int32_t* utt, const float* table, int n_rows, int n_levels,
                             int K, int S, int tr, int noise, const float* uniforms,
-                            uint64_t seed, cudaStream_t st) {
+                            uint64_t seed, const int32_t* known, cudaStream_t st) {
   const int n_tok = n_rows * n_levels;
   const int wpb = 8;
   int grid = (n_tok + wpb - 1) / wpb;
@@ -541,9 +600,13 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
   const bool aligned = (ld % 8 == 0) && ((reinterpret_cast<uintptr_t>(logits) & 15) == 0);
   if (!post_out && aligned && noise != VB200_NOISE_UNIFORMS && K % 256 == 0 && K <= 1024) {
     const T* lg = static_cast<const T*>(logits);
-#define VB_LAUNCH_F(KC, NZ)                                                                      \
-  launch_rc = launch_pdl(posterior_fast_kernel<T, KC, NZ>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, lg, \
-                         static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, n_rows, n_levels, S, tr, lo, hi)
+#define VB_LAUNCH_F(KC, NZ)                                                                                  \
+  launch_rc = known ? launch_pdl(posterior_fast_kernel<T, KC, NZ, true>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, \
+                                 lg, static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, n_rows, n_levels, S, \
+                                 tr, lo, hi, known)                                                                  \
+                    : launch_pdl(posterior_fast_kernel<T, KC, NZ, false>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, \
+                                 lg, static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, n_rows, n_levels, S, \
+                                 tr, lo, hi, known)
 #define VB_LAUNCH_FK(NZ)                                              \
   switch (K / 256) {                                                  \
     case 1: VB_LAUNCH_F(1, NZ); break;                                \
@@ -561,7 +624,7 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
 #define VB_LAUNCH_P(NZ)                                                                        \
   launch_rc = launch_pdl(posterior_sample_kernel<T, NZ>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, post_out,  \
                          static_cast<const T*>(logits), static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, \
-                         n_rows, n_levels, K, S, tr, uniforms, lo, hi)
+                         n_rows, n_levels, K, S, tr, uniforms, lo, hi, known)
   if (noise == VB200_NOISE_PHILOX) VB_LAUNCH_P(VB200_NOISE_PHILOX);
   else if (noise == VB200_NOISE_UNIFORMS) VB_LAUNCH_P(VB200_NOISE_UNIFORMS);
   else VB_LAUNCH_P(VB200_NOISE_GREEDY);
@@ -641,12 +704,12 @@ extern "C" int vb200_q_sample_philox(int32_t* x_out, const int32_t* x0, const in
   return VB200_OK;
 }
 
-extern "C" int vb200_posterior_sample_from_logits(
+extern "C" int vb200_posterior_sample_from_logits_known(
     int32_t* x_out, float* post_out, const void* logits, vb200_dtype logits_dtype,
     int64_t ld_logits, const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
     const int32_t* utt, const float* table, int32_t n_rows, int32_t n_levels, int32_t K,
     int32_t S, vb200_transition tr, vb200_noise noise, const float* uniforms, uint64_t seed,
-    vb200_stream_t stream) {
+    const int32_t* known, vb200_stream_t stream) {
   if (n_rows == 0) return VB200_OK;
   VB_REQUIRE(x_out && logits && x_t && row_utt && t_utt && table, "posterior: null pointer");
   VB_REQUIRE(n_rows >= 0 && n_levels >= 1 && K >= 2 && S >= 1, "posterior: bad sizes");
@@ -658,18 +721,29 @@ extern "C" int vb200_posterior_sample_from_logits(
   switch (logits_dtype) {
     case VB200_F32:
       return launch_posterior<float>(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt, utt,
-                                     table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, st);
+                                     table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known, st);
     case VB200_BF16:
       return launch_posterior<__nv_bfloat16>(x_out, post_out, logits, ld_logits, x_t, row_utt,
                                              t_utt, utt, table, n_rows, n_levels, K, S, tr, noise,
-                                             uniforms, seed, st);
+                                             uniforms, seed, known, st);
     case VB200_F16:
       return launch_posterior<__half>(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt,
                                       utt, table, n_rows, n_levels, K, S, tr, noise, uniforms,
-                                      seed, st);
+                                      seed, known, st);
   }
   set_error("posterior: unknown logits dtype %d", static_cast<int>(logits_dtype));
   return VB200_ERR_INVALID;
+}
+
+extern "C" int vb200_posterior_sample_from_logits(
+    int32_t* x_out, float* post_out, const void* logits, vb200_dtype logits_dtype,
+    int64_t ld_logits, const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+    const int32_t* utt, const float* table, int32_t n_rows, int32_t n_levels, int32_t K,
+    int32_t S, vb200_transition tr, vb200_noise noise, const float* uniforms, uint64_t seed,
+    vb200_stream_t stream) {
+  return vb200_posterior_sample_from_logits_known(x_out, post_out, logits, logits_dtype, ld_logits, x_t, row_utt,
+                                                  t_utt, utt, table, n_rows, n_levels, K, S, tr, noise, uniforms,
+                                                  seed, nullptr, stream);
 }
 
 extern "C" int vb200_step_timesteps(int32_t* t_utt, int32_t B, int32_t delta,

@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
     const int32_t* __restrict__ x_t_all,
     const int32_t* __restrict__ row_utt, const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int K, int Kd, int S, int transition,
-    uint32_t seed_lo, uint32_t seed_hi, uint32_t a_is_f16) {
+    uint32_t seed_lo, uint32_t seed_hi, uint32_t a_is_f16, const int32_t* __restrict__ known) {
   using namespace hs;
   const uint32_t cta_rank = cluster_ctarank();          // 0 = leader of the pair
   extern __shared__ uint8_t smem_raw[];
@@ -174,8 +174,10 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
       int x_t = 0, t = 1;
       uint32_t key1 = 0, gid = 0;
       int b = 0;
+      int kn = -1;                                 // x0 of the token when it is given, else -1
       if (valid) {
         x_t = x_t_all[static_cast<size_t>(grow) * n_levels + level];     // MODE_CE: the target class
+        if (known) kn = known[static_cast<size_t>(grow) * n_levels + level];
         if (NOISE != MODE_CE) {
           b = row_utt[grow];
           t = clamp_timestep(t_utt[b], S);
@@ -324,6 +326,9 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
         if (NOISE == MODE_CE) {
           // -log softmax(logits)[target] = max + ln Z - logit[target]; exactly one half saw the target
           if (valid) loss_out[static_cast<size_t>(grow) * n_levels + level] = m_f + __logf(Z) - (st.e_x + my_x[2]);
+        } else if (kn >= 0) {                            // x0 given: O(1) law of posterior.cuh, logits unused
+          pick = known_pick(post_scalars(table, t, x_t, K, transition), kn, t, K, NOISE == VB200_NOISE_GREEDY,
+                            u01(fin.y), u01(fin.z));
         } else if (t == 0) {
           pick = best_j;                                 // raw logits, no noise (ar_discrete.py:407,413)
         } else {
@@ -361,7 +366,7 @@ template <int NOISE>
 static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_in, const void* W, const float* bias,
                               const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
                               const int32_t* utt, const float* table, int n_rows, int d, int n_levels,
-                              int K, int S, int tr, uint64_t seed, int in_f16, cudaStream_t st) {
+                              int K, int S, int tr, uint64_t seed, int in_f16, const int32_t* known, cudaStream_t st) {
   using namespace hs;
   CUtensorMap ta, tb;
   int rc = cached_tmap(&ta, in_f16 ? VB200_F16 : VB200_BF16, head_in, d, n_rows, static_cast<uint64_t>(d) * 2, BK, BM);
@@ -376,7 +381,7 @@ static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_
   PdlTag pdl_tag(32);
   VB_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(THREADS), SMEM_BYTES, st, 2, ta, tb, x_out, loss_out, bias, x_t, row_utt,
                            t_utt, utt, table, n_rows, n_levels, K, d, S, tr, static_cast<uint32_t>(seed),
-                           static_cast<uint32_t>(seed >> 32), static_cast<uint32_t>(in_f16 ? 1 : 0)));
+                           static_cast<uint32_t>(seed >> 32), static_cast<uint32_t>(in_f16 ? 1 : 0), known));
   VB_CHECK_CUDA(cudaGetLastError());
   return VB200_OK;
 }
@@ -384,12 +389,12 @@ static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias,
                       const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt,
                       const float* table, int n_rows, int d, int n_levels, int K, int S, int tr, int noise,
-                      uint64_t seed, int in_f16, cudaStream_t st) {
+                      uint64_t seed, int in_f16, const int32_t* known, cudaStream_t st) {
   if (noise == VB200_NOISE_GREEDY)
     return launch_head_sample<VB200_NOISE_GREEDY>(x_out, nullptr, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_rows,
-                                                  d, n_levels, K, S, tr, seed, in_f16, st);
+                                                  d, n_levels, K, S, tr, seed, in_f16, known, st);
   return launch_head_sample<VB200_NOISE_PHILOX>(x_out, nullptr, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_rows, d,
-                                                n_levels, K, S, tr, seed, in_f16, st);
+                                                n_levels, K, S, tr, seed, in_f16, known, st);
 }
 
 
@@ -397,7 +402,7 @@ int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const 
 int head_ce_fused(float* loss_out, const void* head_in, const void* W, const float* bias, const int32_t* targets,
                   int n_rows, int d, int n_levels, int K, int in_f16, cudaStream_t st) {
   return launch_head_sample<hs::MODE_CE>(nullptr, loss_out, head_in, W, bias, targets, nullptr, nullptr, nullptr,
-                                         nullptr, n_rows, d, n_levels, K, 1, VB200_UNIFORM, 0, in_f16, st);
+                                         nullptr, n_rows, d, n_levels, K, 1, VB200_UNIFORM, 0, in_f16, nullptr, st);
 }
 
 }  // namespace vb200

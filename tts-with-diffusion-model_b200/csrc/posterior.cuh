@@ -78,6 +78,80 @@ __device__ __forceinline__ int post_greedy(const PostScalars& s, const PostSpeci
   return pick;
 }
 
+// A token whose x0 is given (generate_audio(known_list=...)): the reverse step draws from q(x_s | x_t, x0 = k),
+//   w_j = (Q_{t|s}[j, x_t] + eps) (Qbar_s[k, j] + eps),
+// the ids form of ar_discrete.py:347-375.  Row k of Qbar_s is CUM_BOTH / CUM_KEEP at j = k (k = m or not),
+// CUM_ABSORB at j = m != k and CUM_OFF elsewhere, so at most three classes {x_t, k, m} weigh something of their
+// own and the K - n others share one weight: the law is drawn in O(1) without reading a logit.
+// f1 = Q_{t|s}[j, x_t] + eps and f2 = Qbar_s[k, j] of class j
+__device__ __forceinline__ float2 known_factors(const PostScalars& s, int k, int j) {
+  return make_float2(j == s.x_t ? s.f1_self : s.f1_oth,
+                     j == k ? (j == s.m ? s.a_m : s.a_gen) : (j == s.m ? s.c_m : s.c_gen));
+}
+__device__ __forceinline__ float known_weight(const PostScalars& s, int k, int j) {
+  const float2 f = known_factors(s, k, j);
+  return f.x * (f.y + kEps);
+}
+
+// The special classes of a known token in ascending order, padded with kNone (n of them are classes), their
+// weights (0 for padding) and the weight every other class shares.  Fixed indices only: it stays in registers.
+constexpr int kNone = 0x7fffffff;
+struct KnownLaw {
+  int c[3], n;
+  float w[3], w_gen;
+};
+__device__ __forceinline__ KnownLaw known_law(const PostScalars& s, int k) {
+  KnownLaw l;
+  const int c1 = k != s.x_t ? k : kNone;
+  const int c2 = (s.m >= 0 && s.m != s.x_t && s.m != k) ? s.m : kNone;
+  const int lo = min(s.x_t, c1), hi = max(s.x_t, c1);
+  l.c[0] = min(lo, c2);
+  l.c[1] = max(lo, min(hi, c2));
+  l.c[2] = max(hi, c2);
+  l.n = 1 + (c1 != kNone ? 1 : 0) + (c2 != kNone ? 1 : 0);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) l.w[i] = l.c[i] != kNone ? known_weight(s, k, l.c[i]) : 0.f;
+  l.w_gen = s.f1_oth * (s.c_gen + kEps);
+  return l;
+}
+
+// The reverse step of a known token k.  greedy: the arg max of w, lowest class winning ties (the generic
+// candidate is the lowest class that is not special).  Otherwise a draw from u0 (which group: a special class
+// or the generic ones) and u1 (which generic class, uniformly, special classes skipped).  t == 0 returns k.
+__device__ __forceinline__ int known_pick(const PostScalars& s, int k, int t, int K, bool greedy, float u0, float u1) {
+  if (t == 0) return k;
+  const KnownLaw l = known_law(s, k);
+  const int n_gen = K - l.n;
+  if (greedy) {
+    int g0 = 0;                                          // lowest generic class
+#pragma unroll
+    for (int i = 0; i < 3; ++i) g0 += g0 == l.c[i] ? 1 : 0;
+    float best_w = n_gen > 0 ? l.w_gen : -1.f;
+    int pick = n_gen > 0 ? g0 : kNone;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+      if (l.c[i] != kNone && (l.w[i] > best_w || (l.w[i] == best_w && l.c[i] < pick))) { best_w = l.w[i]; pick = l.c[i]; }
+    return pick;
+  }
+  float target = u0 * (l.w[0] + l.w[1] + l.w[2] + static_cast<float>(n_gen) * l.w_gen);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    if (l.c[i] != kNone && target < l.w[i]) return l.c[i];
+    target -= l.w[i];
+  }
+  if (n_gen <= 0) return l.n == 3 ? l.c[2] : (l.n == 2 ? l.c[1] : l.c[0]);   // rounding at the top end, K == n
+  int j = min(static_cast<int>(u1 * static_cast<float>(n_gen)), n_gen - 1);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) j += j >= l.c[i] ? 1 : 0;  // skip the special classes, ascending
+  return j;
+}
+
+// log w_j of a known token: the posterior logits of the ids form (post_out, Gumbel-max with supplied uniforms)
+__device__ __forceinline__ float known_logit(const PostScalars& s, int k, int j) {
+  const float2 f = known_factors(s, k, j);
+  return logf(f.x) + logf(f.y + kEps);
+}
+
 // Philox counter words of a token's draws: (frame * n_levels + level, global utterance id), which do not depend on
 // how the batch is packed or sharded.  b: the token's utterance, row: its packed response row.
 struct TokenKey { uint32_t tok, gid; };

@@ -52,6 +52,9 @@ def main():
     parser.add_argument("--seed", type=int, default=0)
     parser.add_argument("--steps", type=int, default=None,
                         help="denoise steps of a diffusion first stage, 1 .. n_steps-1 (default: every timestep)")
+    parser.add_argument("--continue-from", type=Path, default=None, metavar="PART.wav",
+                        help="diffusion first stage: keep PART.wav's EnCodec frames as the start of the response and "
+                             "generate the rest, up to --frames frames in all")
     args = parser.parse_args()
 
     try:
@@ -66,10 +69,23 @@ def main():
     proms = to_device(proms, args.device)
     phns = to_device(phns, args.device)
 
+    known_list = None
+    if args.continue_from is not None:
+        if not isinstance(first, Diffusion):
+            raise SystemExit("python -m vall_e: --continue-from needs a diffusion first stage (a Diffusion checkpoint)")
+        prefix = rearrange(qnt.encode_from_file(args.continue_from), "1 l t -> t l")
+        total = args.frames or 350
+        if total <= prefix.shape[0]:
+            raise SystemExit(f"python -m vall_e: --frames ({total}) must exceed the {prefix.shape[0]} frames of "
+                             f"{args.continue_from}")
+        known = torch.full((total, prefix.shape[1]), -1, dtype=torch.long)
+        known[: prefix.shape[0]] = prefix.cpu()
+        known_list = [to_device(known, args.device)]
+
     if isinstance(first, Diffusion):
         lens = [args.frames] if args.frames else None
         resps_list = first.generate_audio(text_list=[phns], proms_list=[proms], resp_lens=lens, seed=args.seed,
-                                          sample_steps=args.steps)
+                                          sample_steps=args.steps, known_list=known_list)
     else:
         nar = _load(args.nar_ckpt, args.device)
         if isinstance(first, DiscreteAR):       # the reference's own D3PM class: level 0 by diffusion, 350 frames

@@ -300,11 +300,11 @@ class DenoiserEngine:
     def reverse_loop(self, lay: BatchLayout, ws: Workspace, x_t: torch.Tensor, table: torch.Tensor,
                      timesteps: int, transition: int, noise: int = L.NOISE_PHILOX, seed: int = 0,
                      uniforms_fn=None, use_graph: bool = True, n_levels: int = 8, trace: list | None = None,
-                     schedule=None, next_t: torch.Tensor | None = None):
+                     schedule=None, next_t: torch.Tensor | None = None, known: torch.Tensor | None = None):
         """One-shot form (tests): x_T -> x_0 in place on x_t int32 (M_resp, n_levels)."""
         ses = Session(self, lay, ws=ws, x_t=x_t)
         ses.run(table, timesteps, transition, noise=noise, seed=seed, uniforms_fn=uniforms_fn,
-                use_graph=use_graph, n_levels=n_levels, trace=trace, schedule=schedule, next_t=next_t)
+                use_graph=use_graph, n_levels=n_levels, trace=trace, schedule=schedule, next_t=next_t, known=known)
         return x_t
 
 
@@ -331,6 +331,14 @@ class Session:
         self.graph_key = None
         self.per_step_launches = 0
         self._next_t = {}
+        self._known = None
+
+    def known_buffer(self) -> torch.Tensor:
+        """The session's int32 (M_resp, n_levels) buffer of given codes (-1 = generate), allocated on first use.
+        Callers fill it per call; its address stays, so a captured step graph that reads it replays."""
+        if self._known is None:
+            self._known = torch.empty_like(self.x_t)
+        return self._known
 
     def signature(self):
         return (tuple(self.lay.t_txt), tuple(self.lay.t_prom), tuple(self.lay.t_resp))
@@ -358,13 +366,17 @@ class Session:
 
     def run(self, table: torch.Tensor, timesteps: int, transition: int, noise: int = L.NOISE_PHILOX,
             seed: int = 0, uniforms_fn=None, use_graph: bool = True, n_levels: int = 8,
-            trace: list | None = None, schedule=None, next_t: torch.Tensor | None = None) -> torch.Tensor:
+            trace: list | None = None, schedule=None, next_t: torch.Tensor | None = None,
+            known: torch.Tensor | None = None) -> torch.Tensor:
         """for t in schedule (default S-1 .. 1; never t = 0, as the reference, ar_discrete.py:750):
         logits = denoiser(x_t, t); x_{sigma(t)} = p_sample(logits, t, x_t), in place on self.x_t, where
         sigma(t) is the next timestep of the schedule (0 after the last).  ``table`` must be the schedule's
         (``d3pm.schedule_table``; ``d3pm.scalar_table`` for the default) and ``next_t`` its int32 (S,)
         successor vector on the device (``successor_tensor``; built here when omitted).
-        uniforms_fn(t) -> float32 (M_resp*n_levels, K) supplies the reference's torch.rand (parity)."""
+        uniforms_fn(t) -> float32 (M_resp*n_levels, K) supplies the reference's torch.rand (parity).
+        ``known``: int32 (M_resp, n_levels) device tensor (``known_buffer``) or None.  A token with known[r, l] = k
+        >= 0 draws every step from q(x_s | x_t, x0 = k) and is set to k once after the last step; -1 draws as
+        usual (vb200_head_posterior_sample_known)."""
         from ..vall_e import d3pm
         if schedule is None:
             schedule = range(timesteps - 1, 0, -1)
@@ -376,10 +388,13 @@ class Session:
         elif next_t.numel() != timesteps:
             raise ValueError(f"next_t has {next_t.numel()} entries, the table {timesteps} timesteps")
         with torch.cuda.device(self.eng.w.device):
-            return self._run(table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels,
-                             trace)
+            self._run(table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace,
+                      known)
+            if known is not None:      # the given codes come back exactly: once per generation, not per step
+                self.x_t.copy_(torch.where(known >= 0, known, self.x_t))
+            return self.x_t
 
-    def _run(self, table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace):
+    def _run(self, table, schedule, next_t, transition, noise, seed, uniforms_fn, use_graph, n_levels, trace, known):
         eng, lay, ws, x_t, t_utt = self.eng, self.lay, self.ws, self.x_t, self.t_utt
         w, dev = eng.w, eng.w.device
         K = w.n_out // n_levels
@@ -389,12 +404,13 @@ class Session:
             if eng.profile is None and not eng.simt:
                 head_in = eng._forward(lay, ws, x_t, t_utt, True, None, False)
                 L.head_posterior_sample(x_t, ws.logits, head_in, w.w_cls, w.b_cls, x_t, lay.resp_row_utt, t_utt,
-                                        lay.utt, table, n_levels, K, transition, noise, uniforms, seed)
+                                        lay.utt, table, n_levels, K, transition, noise, uniforms, seed, known)
                 eng.launches += 0 if L.head_fused(w.d, K, noise) else 1   # the `+= 2` below counts one of them
             else:                 # per-launch timing hooks / CUDA-core validation path: separate calls
                 logits = eng._forward(lay, ws, x_t, t_utt, True, None, True)
                 L.posterior_sample_from_logits(x_t, None, logits, w.n_out, x_t, lay.resp_row_utt, t_utt, lay.utt,
-                                               table, lay.M_resp, n_levels, K, transition, noise, uniforms, seed)
+                                               table, lay.M_resp, n_levels, K, transition, noise, uniforms, seed,
+                                               known)
             L.step_timesteps_to(t_utt, next_t)
             eng.launches += 2
 
@@ -407,7 +423,8 @@ class Session:
                 if trace is not None:
                     trace.append(x_t.clone())
             return x_t
-        key = (table.data_ptr(), next_t.data_ptr(), transition, noise, seed, n_levels)
+        key = (table.data_ptr(), next_t.data_ptr(), transition, noise, seed, n_levels,
+               known.data_ptr() if known is not None else None)
         first = 0
         if self.graph is None or self.graph_key != key:
             # First step eagerly (also warms tensor-map caches and function attributes), then capture

@@ -49,6 +49,13 @@ PROTOTYPES = {
         [_p, _p, C.c_int, _p, C.c_int, _p, _p, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p, _u64,
          _p],
         C.c_int),
+    "vb200_posterior_sample_from_logits_known": (
+        [_p, _p, _p, C.c_int, _i64, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, C.c_int, C.c_int, _p, _u64, _p, _p],
+        C.c_int),
+    "vb200_head_posterior_sample_known": (
+        [_p, _p, C.c_int, _p, C.c_int, _p, _p, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p, _u64,
+         _p, _p],
+        C.c_int),
     "vb200_q_sample_philox": ([_p] * 5 + [_i32, _i32, _i32, C.c_int, _u64, _p], C.c_int),
     "vb200_head_fused": ([_i32, _i32, C.c_int], C.c_int),
     "vb200_head_ce_loss": ([_p, _p, C.c_int, _p, _p, _p, _i32, _i32, _i32, _i32, _p], C.c_int),
@@ -205,23 +212,38 @@ def q_sample_dense(x_out, x0, t_tok, mask, uniforms, log_qbar):
 
 
 def posterior_sample_from_logits(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt, utt, table,
-                                 n_rows, n_levels, K, transition, noise, uniforms=None, seed=0):
-    _check(load().vb200_posterior_sample_from_logits(
+                                 n_rows, n_levels, K, transition, noise, uniforms=None, seed=0, known=None):
+    """``known``: int32 (n_rows, n_levels), -1 = draw as usual, k in [0, K) = the token's x0 is k (the ``_known``
+    entry point); None calls the plain one."""
+    if known is None:
+        _check(load().vb200_posterior_sample_from_logits(
+            ptr(x_out), ptr(post_out), ptr(logits), dtype_code(logits.dtype), ld_logits, ptr(x_t),
+            ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), n_rows, n_levels, K, table.shape[0], transition,
+            noise, ptr(uniforms), seed, stream()), "vb200_posterior_sample_from_logits")
+        return
+    _check(load().vb200_posterior_sample_from_logits_known(
         ptr(x_out), ptr(post_out), ptr(logits), dtype_code(logits.dtype), ld_logits, ptr(x_t),
         ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), n_rows, n_levels, K, table.shape[0], transition,
-        noise, ptr(uniforms), seed, stream()), "vb200_posterior_sample_from_logits")
+        noise, ptr(uniforms), seed, ptr(known), stream()), "vb200_posterior_sample_from_logits_known")
 
 
 def head_posterior_sample(x_out, logits, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_levels, K,
-                          transition, noise, uniforms=None, seed=0):
+                          transition, noise, uniforms=None, seed=0, known=None):
     """classifier + reverse step in one C call: one kernel (reverse step as the GEMM epilogue) when
-    head_fused(), else GEMM into the caller's `logits` scratch (required then) + standalone kernel."""
+    head_fused(), else GEMM into the caller's `logits` scratch (required then) + standalone kernel.
+    ``known`` as in posterior_sample_from_logits."""
     n_rows, d = head_in.shape
-    _check(load().vb200_head_posterior_sample(
-        ptr(x_out), ptr(logits), dtype_code(logits.dtype) if logits is not None else dtype_code(torch.float16),
-        ptr(head_in), act_code(head_in), ptr(W), ptr(bias), n_rows, d,
+    ldt = dtype_code(logits.dtype) if logits is not None else dtype_code(torch.float16)
+    if known is None:
+        _check(load().vb200_head_posterior_sample(
+            ptr(x_out), ptr(logits), ldt, ptr(head_in), act_code(head_in), ptr(W), ptr(bias), n_rows, d,
+            n_levels, K, ptr(x_t), ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), table.shape[0], transition,
+            noise, ptr(uniforms), seed, stream()), "vb200_head_posterior_sample")
+        return
+    _check(load().vb200_head_posterior_sample_known(
+        ptr(x_out), ptr(logits), ldt, ptr(head_in), act_code(head_in), ptr(W), ptr(bias), n_rows, d,
         n_levels, K, ptr(x_t), ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), table.shape[0], transition,
-        noise, ptr(uniforms), seed, stream()), "vb200_head_posterior_sample")
+        noise, ptr(uniforms), seed, ptr(known), stream()), "vb200_head_posterior_sample_known")
 
 
 def q_sample_philox(x_out, x0, t_tok, mask, table, K, transition, seed=0):

@@ -104,7 +104,7 @@ class D3PMOps:
 
     # ------------------------------------------------------------------ reverse step (row P)
     def _posterior(self, model_logits: Tensor, t: Tensor, x: Tensor, noise_mode: int, noise, want_post: bool,
-                   seed: int = 0):
+                   seed: int = 0, known: Tensor | None = None):
         B, W, K = model_logits.shape
         if K != self.num_classes:
             raise ValueError(f"logits have {K} classes, model has {self.num_classes}")
@@ -124,14 +124,23 @@ class D3PMOps:
         uni = noise.to(dev, torch.float32).contiguous() if noise is not None else None
         with torch.cuda.device(dev):
             L.posterior_sample_from_logits(out, post, logits, K, x_t, row_utt, t_utt, utt, self._table(dev),
-                                           B * W, 1, K, _TRANSITIONS[self.transition], noise_mode, uni, seed)
+                                           B * W, 1, K, _TRANSITIONS[self.transition], noise_mode, uni, seed,
+                                           known.to(dev) if known is not None else None)
         return out.view(B, W).long(), (post.view(B, W, K) if want_post else None)
 
     def q_posterior_logits(self, x_start: Tensor, x_t: Tensor, t: Tensor, x_start_logits: bool = True) -> Tensor:
-        """logits of q(x_{t-1} | x_t, p(x_0)) (ar_discrete.py:347-375), fp32 closed form."""
-        if not x_start_logits:
-            raise NotImplementedError("only the logits form used by p_sample is implemented")
-        return self._posterior(x_start, t, x_t, L.NOISE_GREEDY, None, want_post=True)[1]
+        """logits of q(x_{t-1} | x_t, p(x_0)) (ar_discrete.py:347-375), fp32 closed form.  ``x_start_logits=False``:
+        x_start holds the ids of x0 (B, W) and this is q(x_{t-1} | x_t, x0) — the reference's ids branch, through
+        vb200_posterior_sample_from_logits_known with every token known (0 at t == 0, as the reference returns)."""
+        if x_start_logits:
+            return self._posterior(x_start, t, x_t, L.NOISE_GREEDY, None, want_post=True)[1]
+        B, W = x_start.shape
+        K = self.num_classes
+        known = x_start.to(torch.int32).contiguous().view(-1)
+        check_ids(known, K, "q_posterior_logits: x_start")
+        # the logit rows of known tokens are never read: an uninitialised (B, W, K) placeholder fills the argument
+        placeholder = torch.empty(B, W, K, dtype=torch.float16, device=x_start.device)
+        return self._posterior(placeholder, t, x_t, L.NOISE_GREEDY, None, want_post=True, known=known)[1]
 
     def p_sample(self, model_logits: Tensor, t: Tensor, x: Tensor, noise: Tensor | None = None,
                  greedy: bool = False, seed: int | None = None):
@@ -204,7 +213,8 @@ class Diffusion(D3PMOps, Base):
     def generate_audio(self, text_list: list[Tensor], proms_list: list[Tensor], resps_list=None, *,
                        resp_lens: list[int] | None = None, seed: int = 0, greedy: bool = False,
                        uniforms_fn=None, gids=None, use_graph: bool = True, trace: list | None = None,
-                       to_host: bool = False, as_bqt: bool = False, sample_steps: int | None = None):
+                       to_host: bool = False, as_bqt: bool = False, sample_steps: int | None = None,
+                       known_list: list[Tensor] | None = None):
         """x_T -> x_0 for a batch of utterances; returns [LongTensor (t'', 8)].
 
         x_T is all ``mask_id`` for the absorbing transition (ar_discrete.py:699) and uniform random
@@ -219,8 +229,16 @@ class Diffusion(D3PMOps, Base):
         ``as_bqt`` returns ``(LongTensor (B, 8, T_max), [t''])`` instead: the whole batch in the layout
         ``emb/qnt.py:32-49 decode(codes (b q t))`` takes, zero-padded, so the EnCodec stage decodes
         the batch in one call instead of one ``t q -> 1 q t`` utterance at a time (SURVEY §8f.4).
+        ``known_list``: per utterance an integer (t'', 8) tensor of given codes, -1 where a code is to be
+        generated (continuation: a known prefix; span editing: known frames around a span; level-conditional:
+        known levels).  Its lengths define ``resp_lens``.  Known tokens start from the same x_T as the others and
+        draw every step from the exact posterior q(x_s | x_t, x0 = k); the returned codes equal the given ones at
+        every known position (DESIGN.md §5).
         """
         n_steps = self._sample_steps(sample_steps)
+        known = None
+        if known_list is not None:      # checked before the device is touched, like sample_steps
+            known, resp_lens = self._known(known_list, resp_lens, resps_list, len(text_list))
         eng = self.engine()
         dev = eng.w.device
         schedule, table, next_t = self._sampling(dev, n_steps)
@@ -230,6 +248,8 @@ class Diffusion(D3PMOps, Base):
             resp_lens = [350] * len(text_list)
         ses = self._session(text_list, proms_list, resp_lens, gids)
         lay, x_t = ses.lay, ses.x_t
+        if known is not None:
+            known = ses.known_buffer().copy_(known, non_blocking=True)
         if resps_list is not None:
             x_T = torch.cat([r.reshape(len(r), self.n_levels) for r in resps_list]).to(torch.int32)
             check_ids(x_T, self.num_classes, "resps_list (x_T)")
@@ -248,7 +268,7 @@ class Diffusion(D3PMOps, Base):
         noise = L.NOISE_GREEDY if greedy else (L.NOISE_UNIFORMS if uniforms_fn is not None else L.NOISE_PHILOX)
         ses.run(table, self.timesteps, _TRANSITIONS[self.transition], noise=noise, seed=seed,
                 uniforms_fn=uniforms_fn, use_graph=use_graph, n_levels=self.n_levels, trace=trace,
-                schedule=schedule, next_t=next_t)
+                schedule=schedule, next_t=next_t, known=known)
         if as_bqt:        # one (B, 8, T_max) int64 tensor in the EnCodec decoder's layout + the frame counts
             bqt = torch.empty(lay.B, self.n_levels, max(lay.t_resp), dtype=torch.int64, device=dev)
             with torch.cuda.device(dev):
@@ -256,6 +276,27 @@ class Diffusion(D3PMOps, Base):
             return (bqt.cpu() if to_host else bqt), list(lay.t_resp)
         out = x_t.to("cpu", non_blocking=False) if to_host else x_t
         return [r.long() for r in out.split(lay.t_resp, dim=0)]
+
+    def _known(self, known_list, resp_lens, resps_list, B):
+        """(int32 (sum t'', 8) packed given codes, resp_lens) of ``known_list``; ValueError for a wrong count or
+        shape, or lengths that disagree with ``resp_lens`` / ``resps_list``; IndexError for ids outside [-1, K)."""
+        if len(known_list) != B:
+            raise ValueError(f"known_list has {len(known_list)} entries for {B} utterances")
+        for i, k in enumerate(known_list):
+            if not isinstance(k, Tensor) or k.dim() != 2 or k.shape[1] != self.n_levels:
+                raise ValueError(f"known_list[{i}] must be a ({{frames}}, {self.n_levels}) tensor, "
+                                 f"got {tuple(k.shape) if isinstance(k, Tensor) else type(k).__name__}")
+            if k.dtype.is_floating_point or k.dtype == torch.bool or k.dtype.is_complex:
+                raise ValueError(f"known_list[{i}] must hold integer codes, got {k.dtype}")
+        lens = [int(k.shape[0]) for k in known_list]
+        if resp_lens is not None and [int(n) for n in resp_lens] != lens:
+            raise ValueError(f"resp_lens {list(resp_lens)} disagree with the lengths of known_list {lens}")
+        if resps_list is not None and [len(r) for r in resps_list] != lens:
+            raise ValueError(f"resps_list lengths {[len(r) for r in resps_list]} disagree with known_list {lens}")
+        known = torch.cat([k.to(torch.int32) for k in known_list]) if lens else torch.zeros(0, self.n_levels,
+                                                                                            dtype=torch.int32)
+        check_ids(known, self.num_classes, "known_list", lo=-1)
+        return known, lens
 
     # ------------------------------------------------------------------ training forward (SURVEY §8f.3)
     @torch.no_grad()
