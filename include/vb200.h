@@ -223,6 +223,21 @@ int vb200_posterior_sample_from_logits_known(int32_t* x_out, float* post_out, co
                                              vb200_noise noise, const float* uniforms, uint64_t seed,
                                              const int32_t* known, vb200_stream_t stream);
 
+/* P at a sampling temperature: vb200_posterior_sample_from_logits_known plus `temperature` tau (finite, > 0, else
+ * VB200_ERR_INVALID).  p̂(x0) = softmax(logits / tau) enters the posterior in place of softmax(logits), for Philox,
+ * supplied uniforms (post_out then holds the posterior logits on logits / tau) and greedy draws alike.  Not scaled:
+ * t == 0 (the arg max of the raw logits, ar_discrete.py:407,413) and known tokens (their logits are never read).
+ * tau = 1 is vb200_posterior_sample_from_logits_known bit for bit (x * 1.0f is exact); that entry point and the plain
+ * one pass 1. */
+int vb200_posterior_sample_from_logits_temp(int32_t* x_out, float* post_out, const void* logits,
+                                            vb200_dtype logits_dtype, int64_t ld_logits,
+                                            const int32_t* x_t, const int32_t* row_utt,
+                                            const int32_t* t_utt, const int32_t* utt,
+                                            const float* table, int32_t n_rows, int32_t n_levels,
+                                            int32_t K, int32_t S, vb200_transition tr,
+                                            vb200_noise noise, const float* uniforms, uint64_t seed,
+                                            const int32_t* known, float temperature, vb200_stream_t stream);
+
 /* H1 + P in one call (SURVEY.md §8a rows H1 and P; reference base.py:355,440 followed by
  * ar_discrete.py:347-375,401-420): logits = head_in (n_rows, d) x W (n_levels*K, d)^T + bias (both bf16 or both fp16) and
  * the reverse step of vb200_posterior_sample_from_logits on them.
@@ -253,6 +268,33 @@ int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, vb200_dtype 
                                       const int32_t* utt, const float* table, int32_t S,
                                       vb200_transition tr, vb200_noise noise, const float* uniforms,
                                       uint64_t seed, const int32_t* known, vb200_stream_t stream);
+
+/* vb200_head_posterior_sample_known at a sampling temperature, with the semantics of
+ * vb200_posterior_sample_from_logits_temp and the same fused / unfused dispatch.  In the fused kernel the greedy
+ * arg max and t == 0 stay on the raw logits; 1/tau scales the exponent of the streaming softmax. */
+int vb200_head_posterior_sample_temp(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                     const void* head_in, vb200_dtype head_in_dtype, const void* W,
+                                     const float* bias, int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                     const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                     const int32_t* utt, const float* table, int32_t S,
+                                     vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                     uint64_t seed, const int32_t* known, float temperature, vb200_stream_t stream);
+
+/* Classifier + plain categorical draw (the NAR's per-level sampler, reference base.py:491-495
+ * `Categorical(logits / temperature).sample()`): logits = head_in (n_rows, d) x W (K, d)^T + bias, one class per row
+ * drawn from softmax(logits / temperature) and written to x_out[row * ld_out + col]; every other entry of x_out is
+ * left untouched (a NAR pass writes column `level` of the (n_rows, 8) code buffer).  Philox draws are keyed by
+ * (seed, global utterance id, frame * ld_out + col) from the utt records (row_utt maps a row to its utterance), on a
+ * counter stream no D3PM draw uses, so codes do not depend on batch composition or sharding.  Greedy: the arg max
+ * of the raw logits, lowest class wins ties.  Where vb200_head_fused(d, K, noise) holds this is ONE kernel (the draw
+ * is the GEMM's epilogue, `logits` may be NULL); otherwise the logits go through the caller's scratch `logits`
+ * (n_rows, K) of logits_dtype and a one-warp-per-row kernel.  VB200_NOISE_UNIFORMS: VB200_ERR_UNSUPPORTED (the
+ * reference draws with torch.distributions, there is no supplied-noise convention to reproduce); temperature <= 0,
+ * NaN or inf: VB200_ERR_INVALID. */
+int vb200_head_categorical_sample(int32_t* x_out, int64_t ld_out, int32_t col, void* logits, vb200_dtype logits_dtype,
+                                  const void* head_in, vb200_dtype head_in_dtype, const void* W, const float* bias,
+                                  int32_t n_rows, int32_t d, int32_t K, const int32_t* row_utt, const int32_t* utt,
+                                  float temperature, vb200_noise noise, uint64_t seed, vb200_stream_t stream);
 
 /* 1 when vb200_head_posterior_sample runs as one kernel for this configuration (K % 256 == 0,
  * 256 <= K <= 4096, d % 8 == 0, noise != VB200_NOISE_UNIFORMS), else 0.  Host-only call. */

@@ -174,14 +174,19 @@ extern "C" int64_t vb200_workspace_bytes(int64_t M, int64_t M_resp, int32_t d, i
   return total;
 }
 
-extern "C" int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
-                                                 const void* head_in_bf16, vb200_dtype head_in_dtype,
-                                                 const void* W_bf16, const float* bias,
-                                                 int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
-                                                 const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
-                                                 const int32_t* utt, const float* table, int32_t S,
-                                                 vb200_transition tr, vb200_noise noise, const float* uniforms,
-                                                 uint64_t seed, const int32_t* known, vb200_stream_t stream) {
+extern "C" int vb200_head_posterior_sample_temp(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                                const void* head_in_bf16, vb200_dtype head_in_dtype,
+                                                const void* W_bf16, const float* bias,
+                                                int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                                const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                                const int32_t* utt, const float* table, int32_t S,
+                                                vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                                uint64_t seed, const int32_t* known, float temperature,
+                                                vb200_stream_t stream) {
+  if (!vb200::valid_temperature(temperature)) {
+    vb200::set_error("head_posterior_sample: temperature must be finite and > 0, got %g", static_cast<double>(temperature));
+    return VB200_ERR_INVALID;
+  }
   if (head_in_dtype != VB200_BF16 && head_in_dtype != VB200_F16) {
     vb200::set_error("head_posterior_sample: head_in must be bf16 or f16");
     return VB200_ERR_INVALID;
@@ -198,15 +203,28 @@ extern "C" int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, v
     }
     return vb200::head_sample_fused(x_out, head_in_bf16, W_bf16, bias, x_t, row_utt, t_utt, utt, table, n_rows, d,
                              n_levels, K, S, static_cast<int>(tr), static_cast<int>(noise), seed,
-                             head_in_dtype == VB200_F16, known, static_cast<cudaStream_t>(stream));
+                             head_in_dtype == VB200_F16, known, 1.0f / temperature, static_cast<cudaStream_t>(stream));
   }
   const int rc = vb200_gemm_bf16(logits, logits_dtype, head_in_bf16, head_in_dtype, W_bf16, bias, nullptr, n_rows,
                                  n_levels * K, d, VB200_EPI_BIAS, stream);
   if (rc != VB200_OK) return rc;
-  return vb200_posterior_sample_from_logits_known(x_out, nullptr, logits, logits_dtype,
-                                                  static_cast<int64_t>(n_levels) * K, x_t, row_utt, t_utt, utt,
-                                                  table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known,
-                                                  stream);
+  return vb200_posterior_sample_from_logits_temp(x_out, nullptr, logits, logits_dtype,
+                                                 static_cast<int64_t>(n_levels) * K, x_t, row_utt, t_utt, utt,
+                                                 table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known,
+                                                 temperature, stream);
+}
+
+extern "C" int vb200_head_posterior_sample_known(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
+                                                 const void* head_in_bf16, vb200_dtype head_in_dtype,
+                                                 const void* W_bf16, const float* bias,
+                                                 int32_t n_rows, int32_t d, int32_t n_levels, int32_t K,
+                                                 const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+                                                 const int32_t* utt, const float* table, int32_t S,
+                                                 vb200_transition tr, vb200_noise noise, const float* uniforms,
+                                                 uint64_t seed, const int32_t* known, vb200_stream_t stream) {
+  return vb200_head_posterior_sample_temp(x_out, logits, logits_dtype, head_in_bf16, head_in_dtype, W_bf16, bias,
+                                          n_rows, d, n_levels, K, x_t, row_utt, t_utt, utt, table, S, tr, noise,
+                                          uniforms, seed, known, 1.0f, stream);
 }
 
 extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_dtype logits_dtype,
@@ -220,6 +238,59 @@ extern "C" int vb200_head_posterior_sample(int32_t* x_out, void* logits, vb200_d
   return vb200_head_posterior_sample_known(x_out, logits, logits_dtype, head_in_bf16, head_in_dtype, W_bf16, bias,
                                            n_rows, d, n_levels, K, x_t, row_utt, t_utt, utt, table, S, tr, noise,
                                            uniforms, seed, nullptr, stream);
+}
+
+extern "C" int vb200_head_categorical_sample(int32_t* x_out, int64_t ld_out, int32_t col, void* logits,
+                                             vb200_dtype logits_dtype, const void* head_in, vb200_dtype head_in_dtype,
+                                             const void* W, const float* bias, int32_t n_rows, int32_t d, int32_t K,
+                                             const int32_t* row_utt, const int32_t* utt, float temperature,
+                                             vb200_noise noise, uint64_t seed, vb200_stream_t stream) {
+  using namespace vb200;
+  if (noise == VB200_NOISE_UNIFORMS) {
+    set_error("head_categorical_sample: supplied uniforms are not supported (Philox or greedy)");
+    return VB200_ERR_UNSUPPORTED;
+  }
+  if (noise != VB200_NOISE_PHILOX && noise != VB200_NOISE_GREEDY) {
+    set_error("head_categorical_sample: unknown noise mode %d", static_cast<int>(noise));
+    return VB200_ERR_INVALID;
+  }
+  if (!valid_temperature(temperature)) {
+    set_error("head_categorical_sample: temperature must be finite and > 0, got %g", static_cast<double>(temperature));
+    return VB200_ERR_INVALID;
+  }
+  if (n_rows < 0 || d <= 0 || K < 1 || col < 0 || ld_out <= col) {
+    set_error("head_categorical_sample: bad sizes n_rows=%d d=%d K=%d col=%d ld_out=%lld", n_rows, d, K, col,
+              static_cast<long long>(ld_out));
+    return VB200_ERR_INVALID;
+  }
+  if (head_in_dtype != VB200_BF16 && head_in_dtype != VB200_F16) {
+    set_error("head_categorical_sample: head_in must be bf16 or f16");
+    return VB200_ERR_INVALID;
+  }
+  if (n_rows == 0) return VB200_OK;
+  if (!(x_out && head_in && W && bias && row_utt && utt)) {
+    set_error("head_categorical_sample: null pointer");
+    return VB200_ERR_INVALID;
+  }
+  const float inv_temp = 1.0f / temperature;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (vb200_head_fused(d, K, noise)) {                            // one kernel: the draw is the GEMM's epilogue
+    if (reinterpret_cast<uintptr_t>(bias) & 15) {                // the epilogue reads bias as float4
+      set_error("head_categorical_sample: bias must be 16-byte aligned");
+      return VB200_ERR_INVALID;
+    }
+    return head_categorical_fused(x_out, ld_out, col, head_in, W, bias, row_utt, utt, n_rows, d, K,
+                                  static_cast<int>(noise), seed, head_in_dtype == VB200_F16, inv_temp, st);
+  }
+  if (!logits) {
+    set_error("head_categorical_sample: logits scratch (n_rows, K) required when the head is not fused");
+    return VB200_ERR_INVALID;
+  }
+  const int rc = vb200_gemm_bf16(logits, logits_dtype, head_in, head_in_dtype, W, bias, nullptr, n_rows, K, d,
+                                 VB200_EPI_BIAS, stream);
+  if (rc != VB200_OK) return rc;
+  return categorical_from_logits(x_out, ld_out, col, logits, logits_dtype, K, row_utt, utt, n_rows, K,
+                                 static_cast<int>(noise), seed, inv_temp, st);
 }
 
 extern "C" int vb200_head_ce_loss(float* loss, const void* head_in_bf16, vb200_dtype head_in_dtype,

@@ -30,11 +30,21 @@ int cuda_fail(cudaError_t e, const char* what);
 
 int num_sms();
 
+// a sampling temperature the reverse-step and categorical entry points accept: finite and > 0 (NaN fails both)
+inline bool valid_temperature(float t) { return t > 0.f && t <= 3.402823466e+38f; }
+
 // classifier GEMM with the reverse step as its epilogue (head_sample_tcgen05.cu)
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias, const int32_t* x_t,
                       const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt, const float* table,
                       int n_rows, int d, int n_levels, int K, int S, int tr, int noise, uint64_t seed,
-                      int in_f16, const int32_t* known, cudaStream_t st);
+                      int in_f16, const int32_t* known, float inv_temp, cudaStream_t st);
+int head_categorical_fused(int32_t* x_out, int64_t ld_out, int col, const void* head_in, const void* W,
+                           const float* bias, const int32_t* row_utt, const int32_t* utt, int n_rows, int d, int K,
+                           int noise, uint64_t seed, int in_f16, float inv_temp, cudaStream_t st);
+// one categorical draw per row from softmax(logits / tau) for any K, one warp per row (d3pm.cu)
+int categorical_from_logits(int32_t* x_out, int64_t ld_out, int col, const void* logits, vb200_dtype logits_dtype,
+                            int64_t ld_logits, const int32_t* row_utt, const int32_t* utt, int n_rows, int K,
+                            int noise, uint64_t seed, float inv_temp, cudaStream_t st);
 int head_ce_fused(float* loss_out, const void* head_in, const void* W, const float* bias, const int32_t* targets,
                   int n_rows, int d, int n_levels, int K, int in_f16, cudaStream_t st);
 

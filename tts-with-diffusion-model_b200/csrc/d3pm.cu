@@ -224,7 +224,8 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
     int64_t ld_logits, const int32_t* __restrict__ x_t_all, const int32_t* __restrict__ row_utt,
     const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int K, int S, int transition,
-    const float* __restrict__ uniforms, uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known) {
+    const float* __restrict__ uniforms, uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known,
+    float inv_temp) {
   pdl_launch_dependents();
   pdl_wait();                                   // everything below reads / writes activations
   const int warps_per_block = blockDim.x >> 5;
@@ -246,16 +247,17 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
     }
     const T* lrow = logits + static_cast<size_t>(row) * ld_logits + static_cast<size_t>(level) * K;
 
-    // pass 1: row max; pass 2: sum exp (the row is 2-4 KB and stays in L1 between passes)
+    // pass 1: row max; pass 2: sum exp (the row is 2-4 KB and stays in L1 between passes).  p̂(x0) is
+    // softmax(logits * inv_temp); the raw logits are what t == 0 returns (x * 1.0f is exact: tau = 1 is unscaled).
     float mx = -INFINITY;
     if (vec) {
       for (int j0 = lane * 8; j0 < K; j0 += 256) {
         float v[8]; load8<T>(lrow + j0, v);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) mx = fmaxf(mx, v[i]);
+        for (int i = 0; i < 8; ++i) mx = fmaxf(mx, v[i] * inv_temp);
       }
     } else {
-      for (int j = lane; j < K; j += 32) mx = fmaxf(mx, load_logit<T>(lrow, j));
+      for (int j = lane; j < K; j += 32) mx = fmaxf(mx, load_logit<T>(lrow, j) * inv_temp);
     }
     mx = warp_max(mx);
     float sum = 0.f;
@@ -263,10 +265,10 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
       for (int j0 = lane * 8; j0 < K; j0 += 256) {
         float v[8]; load8<T>(lrow + j0, v);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) sum += __expf(v[i] - mx);
+        for (int i = 0; i < 8; ++i) sum += __expf(v[i] * inv_temp - mx);
       }
     } else {
-      for (int j = lane; j < K; j += 32) sum += __expf(load_logit<T>(lrow, j) - mx);
+      for (int j = lane; j < K; j += 32) sum += __expf(load_logit<T>(lrow, j) * inv_temp - mx);
     }
     sum = warp_sum(sum);
     const float inv = 1.0f / sum;
@@ -296,7 +298,7 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const int j = j0 + i;
-          const float pl = post_logit(ps, raw, v[i], __expf(v[i] - mx) * inv, j);
+          const float pl = post_logit(ps, raw, v[i], __expf(v[i] * inv_temp - mx) * inv, j);
           if (prow) prow[j] = pl;
           const float sc = (NOISE != VB200_NOISE_GREEDY && !raw) ? pl + g[i] : pl;
           best_update(best, sc, j);
@@ -305,7 +307,7 @@ __global__ void __launch_bounds__(256) posterior_sample_kernel(
     } else {
       for (int j = lane; j < K; j += 32) {
         const float l = load_logit<T>(lrow, j);
-        const float pl = post_logit(ps, raw, l, __expf(l - mx) * inv, j);
+        const float pl = post_logit(ps, raw, l, __expf(l * inv_temp - mx) * inv, j);
         if (prow) prow[j] = pl;
         float sc = pl;
         if (NOISE == VB200_NOISE_PHILOX && !raw) {
@@ -386,13 +388,16 @@ __device__ __forceinline__ float cvt1(Raw1<__nv_bfloat16> r) { return __bfloat16
 // while token k is reduced.
 // KNOWN: `known` (x0 given for some tokens) is read; a template flag, so that without it the kernel is the
 // register-tight loop it was (a runtime branch costs spills at KC = 4).
+// inv_temp = 1/tau: p̂(x0) = softmax(logits / tau).  A logit only enters an exponent exp2((l - max) * log2 e), so
+// 1/tau is folded into that factor and the max and arg max (greedy, t == 0) stay on the raw logits.  tau = 1
+// multiplies by exactly 1.0f: the unscaled arithmetic bit for bit.
 template <typename T, int KC, int NOISE, bool KNOWN>
 __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
     int32_t* __restrict__ x_out, const T* __restrict__ logits, int64_t ld_logits,
     const int32_t* __restrict__ x_t_all, const int32_t* __restrict__ row_utt,
     const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int S, int transition,
-    uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known) {
+    uint32_t seed_lo, uint32_t seed_hi, const int32_t* __restrict__ known, float inv_temp) {
   constexpr int K = KC * 256;
   pdl_launch_dependents();
   pdl_wait();                                   // everything below reads / writes activations
@@ -487,13 +492,13 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
         }
         top.v = warp_max(fmaxf(fmaxf(m0, m1), fmaxf(m2, m3)));
       }
-      const float mx = top.v;
       if (t == 0) {
         if (lane == 0) x_out[tok] = top.j;
         continue;
       }
-      const float mx_l2 = -mx * kLog2e;
-      const uint64_t l2e2 = pack2(kLog2e, kLog2e), mxl2 = pack2(mx_l2, mx_l2);
+      const float l2e = kLog2e * inv_temp;
+      const float mx_l2 = -top.v * l2e;
+      const uint64_t l2e2 = pack2(l2e, l2e), mxl2 = pack2(mx_l2, mx_l2);
       float part[KC];                                       // per-lane partial sums of e_j, one per 8-chunk
       float lane_sum = 0.f;
 #pragma unroll
@@ -520,8 +525,8 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
         const float n = __shfl_up_sync(kFull, incl, o);
         if (lane >= o) incl += n;
       }
-      const float e_x = exp2f_fast(fmaf(l_x, kLog2e, mx_l2));
-      const float e_m = exp2f_fast(fmaf(l_m, kLog2e, mx_l2));
+      const float e_x = exp2f_fast(fmaf(l_x, l2e, mx_l2));
+      const float e_m = exp2f_fast(fmaf(l_m, l2e, mx_l2));
       const float Z = __shfl_sync(kFull, incl, 31);
       const float invZ = 1.0f / Z;
 
@@ -534,7 +539,7 @@ __global__ void __launch_bounds__(256, 3) posterior_fast_kernel(
       const PostSpecial w = post_special(ps, e_x, e_m, invZ, coef, cst);
       int pick;
       if (NOISE == VB200_NOISE_GREEDY) {
-        pick = post_greedy(ps, w, fmaf(exp2f_fast(fmaf(top.v, kLog2e, mx_l2)), coef, cst), top.j);
+        pick = post_greedy(ps, w, fmaf(exp2f_fast(fmaf(top.v, l2e, mx_l2)), coef, cst), top.j);
       } else {
         const uint32_t rnd = __shfl_sync(kFull, my_rnd, k);
         const float w_generic = fmaf(coef, Z, static_cast<float>(K) * cst);
@@ -588,7 +593,7 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
                             const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
                             const int32_t* utt, const float* table, int n_rows, int n_levels,
                             int K, int S, int tr, int noise, const float* uniforms,
-                            uint64_t seed, const int32_t* known, cudaStream_t st) {
+                            uint64_t seed, const int32_t* known, float inv_temp, cudaStream_t st) {
   const int n_tok = n_rows * n_levels;
   const int wpb = 8;
   int grid = (n_tok + wpb - 1) / wpb;
@@ -603,10 +608,10 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
 #define VB_LAUNCH_F(KC, NZ)                                                                                  \
   launch_rc = known ? launch_pdl(posterior_fast_kernel<T, KC, NZ, true>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, \
                                  lg, static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, n_rows, n_levels, S, \
-                                 tr, lo, hi, known)                                                                  \
+                                 tr, lo, hi, known, inv_temp)                                                        \
                     : launch_pdl(posterior_fast_kernel<T, KC, NZ, false>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, \
                                  lg, static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, n_rows, n_levels, S, \
-                                 tr, lo, hi, known)
+                                 tr, lo, hi, known, inv_temp)
 #define VB_LAUNCH_FK(NZ)                                              \
   switch (K / 256) {                                                  \
     case 1: VB_LAUNCH_F(1, NZ); break;                                \
@@ -624,12 +629,98 @@ static int launch_posterior(int32_t* x_out, float* post_out, const void* logits,
 #define VB_LAUNCH_P(NZ)                                                                        \
   launch_rc = launch_pdl(posterior_sample_kernel<T, NZ>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, post_out,  \
                          static_cast<const T*>(logits), static_cast<int64_t>(ld), x_t, row_utt, t_utt, utt, table, \
-                         n_rows, n_levels, K, S, tr, uniforms, lo, hi, known)
+                         n_rows, n_levels, K, S, tr, uniforms, lo, hi, known, inv_temp)
   if (noise == VB200_NOISE_PHILOX) VB_LAUNCH_P(VB200_NOISE_PHILOX);
   else if (noise == VB200_NOISE_UNIFORMS) VB_LAUNCH_P(VB200_NOISE_UNIFORMS);
   else VB_LAUNCH_P(VB200_NOISE_GREEDY);
 #undef VB_LAUNCH_P
   VB_CHECK_CUDA(launch_rc);
+  VB_CHECK_CUDA(cudaGetLastError());
+  return VB200_OK;
+}
+
+// ---------------------------------------------------------------- plain categorical draw (NAR levels)
+// One class per row from softmax(logits / tau), for the K the fused classifier head does not take: one warp per
+// row, lane i owns the contiguous classes [i*per, (i+1)*per), and the code is the inverse CDF of one Philox uniform
+// (the warp scan of the lane sums finds the lane, the lane walks its classes), as posterior_fast_kernel draws.
+// Greedy: the arg max of the raw logits, lowest class wins ties.  The code goes to x_out[row * ld_out + col]; the
+// Philox counter (CAT_STREAM_1, frame * 8 + level, global utterance id, 0) is used by no D3PM draw.
+constexpr uint32_t CAT_STREAM_1 = 0xCA710000u;
+template <typename T, int NOISE>
+__global__ void __launch_bounds__(256) categorical_kernel(
+    int32_t* __restrict__ x_out, int64_t ld_out, int col, const T* __restrict__ logits, int64_t ld_logits,
+    const int32_t* __restrict__ row_utt, const int32_t* __restrict__ utt, int n_rows, int K, float inv_temp,
+    uint32_t seed_lo, uint32_t seed_hi) {
+  pdl_launch_dependents();
+  pdl_wait();                                   // everything below reads / writes activations
+  const int warps_per_block = blockDim.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const int per = (K + 31) / 32;
+  const int j0 = min(lane * per, K), j1 = min(j0 + per, K);
+  for (int row = blockIdx.x * warps_per_block + (threadIdx.x >> 5); row < n_rows;
+       row += gridDim.x * warps_per_block) {
+    const T* lrow = logits + static_cast<size_t>(row) * ld_logits;
+    int pick;
+    if (NOISE == VB200_NOISE_GREEDY) {
+      Best best{-INFINITY, 0x7fffffff};
+      for (int j = j0; j < j1; ++j) best_update(best, load_logit<T>(lrow, j), j);
+      pick = warp_best(best).j;
+    } else {
+      float mx = -INFINITY;
+      for (int j = j0; j < j1; ++j) mx = fmaxf(mx, load_logit<T>(lrow, j) * inv_temp);
+      mx = warp_max(mx);
+      float lane_sum = 0.f;
+      for (int j = j0; j < j1; ++j) lane_sum += __expf(load_logit<T>(lrow, j) * inv_temp - mx);
+      float incl = lane_sum;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const float n = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += n;
+      }
+      const float Z = __shfl_sync(0xffffffffu, incl, 31);
+      const TokenKey key = token_key(utt, row_utt[row], row, col, static_cast<int>(ld_out));
+      const uint4 r = Philox{seed_lo, seed_hi}(CAT_STREAM_1, key.tok, key.gid, 0u);
+      const float target = u01(r.x) * Z;
+      const unsigned ball = __ballot_sync(0xffffffffu, target < incl && j1 > j0);
+      const int last = (K - 1) / per;                // last lane that owns a class: rounding at the top end
+      const int src = ball ? __ffs(ball) - 1 : last;
+      float run = incl - lane_sum;                   // mass before this lane's classes
+      int idx = j0;
+      for (int j = j0; j + 1 < j1; ++j) {            // prefix sums are monotone: count those <= target
+        run += __expf(load_logit<T>(lrow, j) * inv_temp - mx);
+        idx += target >= run ? 1 : 0;
+      }
+      pick = __shfl_sync(0xffffffffu, idx, src);
+    }
+    if (lane == 0) x_out[static_cast<size_t>(row) * ld_out + col] = pick;
+  }
+}
+
+int categorical_from_logits(int32_t* x_out, int64_t ld_out, int col, const void* logits, vb200_dtype logits_dtype,
+                            int64_t ld_logits, const int32_t* row_utt, const int32_t* utt, int n_rows, int K,
+                            int noise, uint64_t seed, float inv_temp, cudaStream_t st) {
+  const int wpb = 8;
+  int grid = (n_rows + wpb - 1) / wpb;
+  const int cap = num_sms() * 8 * 4;
+  if (grid > cap) grid = cap;
+  const uint32_t lo = static_cast<uint32_t>(seed), hi = static_cast<uint32_t>(seed >> 32);
+  cudaError_t rc = cudaSuccess;
+#define VB_LAUNCH_C(T)                                                                                               \
+  rc = noise == VB200_NOISE_GREEDY                                                                                   \
+           ? launch_pdl(categorical_kernel<T, VB200_NOISE_GREEDY>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, ld_out, \
+                        col, static_cast<const T*>(logits), ld_logits, row_utt, utt, n_rows, K, inv_temp, lo, hi)     \
+           : launch_pdl(categorical_kernel<T, VB200_NOISE_PHILOX>, dim3(grid), dim3(wpb * 32), 0, st, 1, x_out, ld_out, \
+                        col, static_cast<const T*>(logits), ld_logits, row_utt, utt, n_rows, K, inv_temp, lo, hi)
+  switch (logits_dtype) {
+    case VB200_F32: VB_LAUNCH_C(float); break;
+    case VB200_BF16: VB_LAUNCH_C(__nv_bfloat16); break;
+    case VB200_F16: VB_LAUNCH_C(__half); break;
+    default:
+      set_error("categorical: unknown logits dtype %d", static_cast<int>(logits_dtype));
+      return VB200_ERR_INVALID;
+  }
+#undef VB_LAUNCH_C
+  VB_CHECK_CUDA(rc);
   VB_CHECK_CUDA(cudaGetLastError());
   return VB200_OK;
 }
@@ -704,12 +795,15 @@ extern "C" int vb200_q_sample_philox(int32_t* x_out, const int32_t* x0, const in
   return VB200_OK;
 }
 
-extern "C" int vb200_posterior_sample_from_logits_known(
+extern "C" int vb200_posterior_sample_from_logits_temp(
     int32_t* x_out, float* post_out, const void* logits, vb200_dtype logits_dtype,
     int64_t ld_logits, const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
     const int32_t* utt, const float* table, int32_t n_rows, int32_t n_levels, int32_t K,
     int32_t S, vb200_transition tr, vb200_noise noise, const float* uniforms, uint64_t seed,
-    const int32_t* known, vb200_stream_t stream) {
+    const int32_t* known, float temperature, vb200_stream_t stream) {
+  VB_REQUIRE(valid_temperature(temperature), "posterior: temperature must be finite and > 0, got %g",
+             static_cast<double>(temperature));
+  const float inv_temp = 1.0f / temperature;
   if (n_rows == 0) return VB200_OK;
   VB_REQUIRE(x_out && logits && x_t && row_utt && t_utt && table, "posterior: null pointer");
   VB_REQUIRE(n_rows >= 0 && n_levels >= 1 && K >= 2 && S >= 1, "posterior: bad sizes");
@@ -721,18 +815,29 @@ extern "C" int vb200_posterior_sample_from_logits_known(
   switch (logits_dtype) {
     case VB200_F32:
       return launch_posterior<float>(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt, utt,
-                                     table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known, st);
+                                     table, n_rows, n_levels, K, S, tr, noise, uniforms, seed, known, inv_temp, st);
     case VB200_BF16:
       return launch_posterior<__nv_bfloat16>(x_out, post_out, logits, ld_logits, x_t, row_utt,
                                              t_utt, utt, table, n_rows, n_levels, K, S, tr, noise,
-                                             uniforms, seed, known, st);
+                                             uniforms, seed, known, inv_temp, st);
     case VB200_F16:
       return launch_posterior<__half>(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt,
                                       utt, table, n_rows, n_levels, K, S, tr, noise, uniforms,
-                                      seed, known, st);
+                                      seed, known, inv_temp, st);
   }
   set_error("posterior: unknown logits dtype %d", static_cast<int>(logits_dtype));
   return VB200_ERR_INVALID;
+}
+
+extern "C" int vb200_posterior_sample_from_logits_known(
+    int32_t* x_out, float* post_out, const void* logits, vb200_dtype logits_dtype,
+    int64_t ld_logits, const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
+    const int32_t* utt, const float* table, int32_t n_rows, int32_t n_levels, int32_t K,
+    int32_t S, vb200_transition tr, vb200_noise noise, const float* uniforms, uint64_t seed,
+    const int32_t* known, vb200_stream_t stream) {
+  return vb200_posterior_sample_from_logits_temp(x_out, post_out, logits, logits_dtype, ld_logits, x_t, row_utt,
+                                                 t_utt, utt, table, n_rows, n_levels, K, S, tr, noise, uniforms,
+                                                 seed, known, 1.0f, stream);
 }
 
 extern "C" int vb200_posterior_sample_from_logits(

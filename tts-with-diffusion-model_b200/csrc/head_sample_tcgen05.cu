@@ -39,12 +39,19 @@ constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_WARPS * 32 * ROW_BYTES + B
                            1024 /*align slack*/ + 256 /*barriers*/;
 constexpr uint32_t TMEM_COLS = 512;
 constexpr int MODE_CE = 100;                    // epilogue = cross-entropy against target classes (no sampling)
+// Philox stream of the plain categorical draws (CAT): no D3PM draw uses a counter word 0 in [0xCA700000, 0xCA7002ff]
+constexpr uint32_t CAT_STREAM = 0xCA700000u;
 }  // namespace hs
 
 __device__ __forceinline__ void hs_bar_sync(int id, int n_threads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n_threads) : "memory");
 }
 
+// Temperature: the draws are from softmax(logits / tau).  A logit only ever enters through an exponent
+// exp2((l - max) * log2 e), so 1/tau is folded into that factor, l2e = log2 e / tau, and every max, including the
+// arg max (greedy, t == 0), stays on the raw logits.  tau = 1 multiplies by exactly 1.0f: the unscaled arithmetic
+// bit for bit.
+//
 // per-token streaming state of one thread (one accumulator row, one half of each tile's columns)
 struct HsState {
   float m, Z;            // running max of the logits seen (natural log units) and mass relative to it
@@ -55,14 +62,18 @@ struct HsState {
   int win_col;           // first class of the candidate chunk
 };
 
-template <int NOISE>
+// CAT: the plain categorical draw of one class per (row, head) from softmax(logits / tau) (NAR levels): the
+// reservoir candidates of the two halves merged as the cA branch of the mixture does, no table, timestep or x_t.
+// Codes go to x_out[row * ld_out + col + level]; a D3PM step writes (row, level) with ld_out = n_levels, col = 0.
+template <int NOISE, bool CAT = false>
 __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
     const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
     int32_t* __restrict__ x_out, float* __restrict__ loss_out, const float* __restrict__ bias,
     const int32_t* __restrict__ x_t_all,
     const int32_t* __restrict__ row_utt, const int32_t* __restrict__ t_utt, const int32_t* __restrict__ utt,
     const float* __restrict__ table, int n_rows, int n_levels, int K, int Kd, int S, int transition,
-    uint32_t seed_lo, uint32_t seed_hi, uint32_t a_is_f16, const int32_t* __restrict__ known) {
+    uint32_t seed_lo, uint32_t seed_hi, uint32_t a_is_f16, const int32_t* __restrict__ known, float inv_temp,
+    int ld_out, int col_out) {
   using namespace hs;
   const uint32_t cta_rank = cluster_ctarank();          // 0 = leader of the pair
   extern __shared__ uint8_t smem_raw[];
@@ -165,6 +176,8 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
     float* my_x = xchg + r_cta * XCHG_WORDS;
     const int m_abs = transition == VB200_ABSORBING ? K / 2 : -1;
     const Philox ph{seed_lo, seed_hi};
+    const float l2e = kLog2e * inv_temp;
+    const uint32_t stream0 = CAT ? CAT_STREAM : 0xC0DF0000u;
     int it = 0;
     for (int item = item0; item < num_items; item += item_stride) {
       const int m_blk = item / n_levels, level = item - m_blk * n_levels;
@@ -176,17 +189,18 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
       int b = 0;
       int kn = -1;                                 // x0 of the token when it is given, else -1
       if (valid) {
-        x_t = x_t_all[static_cast<size_t>(grow) * n_levels + level];     // MODE_CE: the target class
+        if (!CAT) x_t = x_t_all[static_cast<size_t>(grow) * n_levels + level];     // MODE_CE: the target class
         if (known) kn = known[static_cast<size_t>(grow) * n_levels + level];
         if (NOISE != MODE_CE) {
           b = row_utt[grow];
-          t = clamp_timestep(t_utt[b], S);
-          const TokenKey key = token_key(utt, b, grow, level, n_levels);
+          if (!CAT) t = clamp_timestep(t_utt[b], S);
+          const TokenKey key = token_key(utt, b, grow, col_out + level, ld_out);   // CAT: frame * 8 + NAR level
           key1 = key.tok;
           gid = key.gid;
         }
       }
-      const bool need_arg = NOISE == VB200_NOISE_GREEDY || (NOISE != MODE_CE && t == 0);
+      if (CAT) t = 0;                               // fourth Philox word; a CAT draw has no timestep
+      const bool need_arg = NOISE == VB200_NOISE_GREEDY || (!CAT && NOISE != MODE_CE && t == 0);
       HsState st{-INFINITY, 0.f, 0.f, 0.f, 0.f, 0.f, -INFINITY, 0x7fffffff, 0};
       float win[32];                            // weights of the candidate chunk (local memory: written rarely)
 #pragma unroll
@@ -200,7 +214,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
         const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + as * BN + half * 128;
         // four reservoir decisions per tile from one Philox call (stream 1 + half, counter = tile)
         uint4 rnd = make_uint4(0, 0, 0, 0);
-        if (NOISE == VB200_NOISE_PHILOX) rnd = ph(0xC0DF0000u + (half << 8) + q, key1, gid, t);
+        if (NOISE == VB200_NOISE_PHILOX) rnd = ph(stream0 + (half << 8) + q, key1, gid, t);
         const uint32_t rw[4] = {rnd.x, rnd.y, rnd.z, rnd.w};
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
@@ -237,10 +251,10 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
               st.e_x = *reinterpret_cast<const float*>(my_row + (((dxt >> 2) ^ sw) << 4) + (dxt & 3) * 4);
           }
           const float m_new = fmaxf(st.m, cmax);
-          st.Z *= exp2f_fast((st.m - m_new) * kLog2e);            // 0 on the first chunk (m = -inf)
+          st.Z *= exp2f_fast((st.m - m_new) * l2e);               // 0 on the first chunk (m = -inf)
           st.m = m_new;
-          const float mneg = -m_new * kLog2e;
-          const uint64_t l2e2 = pack2(kLog2e, kLog2e), mneg2 = pack2(mneg, mneg);
+          const float mneg = -m_new * l2e;
+          const uint64_t l2e2 = pack2(l2e, l2e), mneg2 = pack2(mneg, mneg);
           uint64_t acc = 0ull;
 #pragma unroll
           for (int i = 0; i < 32; i += 2) {
@@ -254,7 +268,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
           unpack2(acc, a0, a1);
           const float s_c = a0 + a1;
           st.Z += s_c;
-          if (NOISE != MODE_CE) {
+          if (NOISE != MODE_CE && !CAT) {
             // the chunk's weights go to this thread's staging row: class x_t is read back from it
 #pragma unroll
             for (int k = 0; k < 8; ++k)
@@ -287,7 +301,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
       uint4 fin = make_uint4(0, 0, 0, 0);
       int cand = st.win_col;
       if (NOISE == VB200_NOISE_PHILOX) {
-        fin = ph(0xC0DF0000u + (half << 8) + 0xff, key1, gid, t);
+        fin = ph(stream0 + (half << 8) + 0xff, key1, gid, t);
         float tot = 0.f;
 #pragma unroll
         for (int i = 0; i < 32; ++i) tot += win[i];
@@ -309,11 +323,11 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
       if (half == 0) {
         const float m_b = my_x[0], Z_b = my_x[1];
         const float m_f = fmaxf(st.m, m_b);
-        const float Za = st.Z * exp2f_fast((st.m - m_f) * kLog2e), Zb = Z_b * exp2f_fast((m_b - m_f) * kLog2e);
+        const float Za = st.Z * exp2f_fast((st.m - m_f) * l2e), Zb = Z_b * exp2f_fast((m_b - m_f) * l2e);
         const float Z = Za + Zb, invZ = 1.0f / Z;
         // class x_t / m: whichever half saw it (weights were relative to the max at that time)
-        const float e_x = st.e_x * exp2f_fast((st.m_x - m_f) * kLog2e) + my_x[2] * exp2f_fast((my_x[3] - m_f) * kLog2e);
-        const float e_m = st.e_m * exp2f_fast((st.m_m - m_f) * kLog2e) + my_x[4] * exp2f_fast((my_x[5] - m_f) * kLog2e);
+        const float e_x = st.e_x * exp2f_fast((st.m_x - m_f) * l2e) + my_x[2] * exp2f_fast((my_x[3] - m_f) * l2e);
+        const float e_m = st.e_m * exp2f_fast((st.m_m - m_f) * l2e) + my_x[4] * exp2f_fast((my_x[5] - m_f) * l2e);
         float best = st.best;
         int best_j = st.best_j;
         {
@@ -324,8 +338,10 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
         const int cand_b = __float_as_int(my_x[8]);
         int pick = 0;
         if (NOISE == MODE_CE) {
-          // -log softmax(logits)[target] = max + ln Z - logit[target]; exactly one half saw the target
+          // -log softmax(logits)[target] = max + ln Z - logit[target]; exactly one half saw the target (tau = 1)
           if (valid) loss_out[static_cast<size_t>(grow) * n_levels + level] = m_f + __logf(Z) - (st.e_x + my_x[2]);
+        } else if (CAT) {                                // softmax(logits / tau): merge the two candidates
+          pick = NOISE == VB200_NOISE_GREEDY ? best_j : ((u01(fin.y) * Z < Zb) ? cand_b : cand);
         } else if (kn >= 0) {                            // x0 given: O(1) law of posterior.cuh, logits unused
           pick = known_pick(post_scalars(table, t, x_t, K, transition), kn, t, K, NOISE == VB200_NOISE_GREEDY,
                             u01(fin.y), u01(fin.z));
@@ -337,7 +353,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
           const float coef = cA * invZ;
           const PostSpecial w = post_special(ps, e_x, e_m, invZ, coef, cst);
           if (NOISE == VB200_NOISE_GREEDY) {
-            pick = post_greedy(ps, w, fmaf(exp2f_fast((best - m_f) * kLog2e), coef, cst), best_j);
+            pick = post_greedy(ps, w, fmaf(exp2f_fast((best - m_f) * l2e), coef, cst), best_j);
           } else {
             const float w_uni = static_cast<float>(K) * cst;
             const float target = u01(fin.y) * (cA + w_uni + w.dx + w.dm);
@@ -347,7 +363,7 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
             else pick = (u01(fin.w) * Z < Zb) ? cand_b : cand;     // softmax(logits): merge the two candidates
           }
         }
-        if (NOISE != MODE_CE && valid) x_out[static_cast<size_t>(grow) * n_levels + level] = pick;
+        if (NOISE != MODE_CE && valid) x_out[static_cast<size_t>(grow) * ld_out + col_out + level] = pick;
       }
       hs_bar_sync(1 + quad, 64);                        // half 1 may overwrite its exchange words again
     }
@@ -362,11 +378,12 @@ __global__ void __launch_bounds__(hs::THREADS, 1) head_sample_kernel(
   }
 }
 
-template <int NOISE>
+template <int NOISE, bool CAT = false>
 static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_in, const void* W, const float* bias,
                               const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt,
                               const int32_t* utt, const float* table, int n_rows, int d, int n_levels,
-                              int K, int S, int tr, uint64_t seed, int in_f16, const int32_t* known, cudaStream_t st) {
+                              int K, int S, int tr, uint64_t seed, int in_f16, const int32_t* known, float inv_temp,
+                              int ld_out, int col_out, cudaStream_t st) {
   using namespace hs;
   CUtensorMap ta, tb;
   int rc = cached_tmap(&ta, in_f16 ? VB200_F16 : VB200_BF16, head_in, d, n_rows, static_cast<uint64_t>(d) * 2, BK, BM);
@@ -376,12 +393,13 @@ static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_
   const int items = ((n_rows + 2 * BM - 1) / (2 * BM)) * n_levels;
   const int groups = num_sms() / 2;
   const int grid = (items < groups ? items : groups) * 2;
-  auto kern = head_sample_kernel<NOISE>;
+  auto kern = head_sample_kernel<NOISE, CAT>;
   VB_CONFIGURE_SMEM(kern, SMEM_BYTES);
   PdlTag pdl_tag(32);
   VB_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(THREADS), SMEM_BYTES, st, 2, ta, tb, x_out, loss_out, bias, x_t, row_utt,
                            t_utt, utt, table, n_rows, n_levels, K, d, S, tr, static_cast<uint32_t>(seed),
-                           static_cast<uint32_t>(seed >> 32), static_cast<uint32_t>(in_f16 ? 1 : 0), known));
+                           static_cast<uint32_t>(seed >> 32), static_cast<uint32_t>(in_f16 ? 1 : 0), known, inv_temp,
+                           ld_out, col_out));
   VB_CHECK_CUDA(cudaGetLastError());
   return VB200_OK;
 }
@@ -389,12 +407,25 @@ static int launch_head_sample(int32_t* x_out, float* loss_out, const void* head_
 int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const float* bias,
                       const int32_t* x_t, const int32_t* row_utt, const int32_t* t_utt, const int32_t* utt,
                       const float* table, int n_rows, int d, int n_levels, int K, int S, int tr, int noise,
-                      uint64_t seed, int in_f16, const int32_t* known, cudaStream_t st) {
+                      uint64_t seed, int in_f16, const int32_t* known, float inv_temp, cudaStream_t st) {
   if (noise == VB200_NOISE_GREEDY)
     return launch_head_sample<VB200_NOISE_GREEDY>(x_out, nullptr, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_rows,
-                                                  d, n_levels, K, S, tr, seed, in_f16, known, st);
+                                                  d, n_levels, K, S, tr, seed, in_f16, known, inv_temp, n_levels, 0, st);
   return launch_head_sample<VB200_NOISE_PHILOX>(x_out, nullptr, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_rows, d,
-                                                n_levels, K, S, tr, seed, in_f16, known, st);
+                                                n_levels, K, S, tr, seed, in_f16, known, inv_temp, n_levels, 0, st);
+}
+
+// one categorical draw per row from softmax((head_in W^T + bias) / tau), written to x_out[row * ld_out + col]
+int head_categorical_fused(int32_t* x_out, int64_t ld_out, int col, const void* head_in, const void* W,
+                           const float* bias, const int32_t* row_utt, const int32_t* utt, int n_rows, int d, int K,
+                           int noise, uint64_t seed, int in_f16, float inv_temp, cudaStream_t st) {
+  if (noise == VB200_NOISE_GREEDY)
+    return launch_head_sample<VB200_NOISE_GREEDY, true>(x_out, nullptr, head_in, W, bias, nullptr, row_utt, nullptr, utt,
+                                                        nullptr, n_rows, d, 1, K, 1, VB200_UNIFORM, seed, in_f16, nullptr,
+                                                        inv_temp, static_cast<int>(ld_out), col, st);
+  return launch_head_sample<VB200_NOISE_PHILOX, true>(x_out, nullptr, head_in, W, bias, nullptr, row_utt, nullptr, utt,
+                                                      nullptr, n_rows, d, 1, K, 1, VB200_UNIFORM, seed, in_f16, nullptr,
+                                                      inv_temp, static_cast<int>(ld_out), col, st);
 }
 
 
@@ -402,7 +433,8 @@ int head_sample_fused(int32_t* x_out, const void* head_in, const void* W, const 
 int head_ce_fused(float* loss_out, const void* head_in, const void* W, const float* bias, const int32_t* targets,
                   int n_rows, int d, int n_levels, int K, int in_f16, cudaStream_t st) {
   return launch_head_sample<hs::MODE_CE>(nullptr, loss_out, head_in, W, bias, targets, nullptr, nullptr, nullptr,
-                                         nullptr, n_rows, d, n_levels, K, 1, VB200_UNIFORM, 0, in_f16, nullptr, st);
+                                         nullptr, n_rows, d, n_levels, K, 1, VB200_UNIFORM, 0, in_f16, nullptr, 1.0f,
+                                         n_levels, 0, st);
 }
 
 }  // namespace vb200

@@ -55,6 +55,11 @@ def main():
     parser.add_argument("--continue-from", type=Path, default=None, metavar="PART.wav",
                         help="diffusion first stage: keep PART.wav's EnCodec frames as the start of the response and "
                              "generate the rest, up to --frames frames in all")
+    parser.add_argument("--temperature", type=float, default=1.0,
+                        help="sampling temperature of a diffusion first stage or ar_discrete model: the reverse steps "
+                             "draw from softmax(logits / T) (default 1.0)")
+    parser.add_argument("--nar-temperature", type=float, default=0.2,
+                        help="sampling temperature of the NAR levels 1-7 (default 0.2, as the reference)")
     args = parser.parse_args()
 
     try:
@@ -85,15 +90,16 @@ def main():
     if isinstance(first, Diffusion):
         lens = [args.frames] if args.frames else None
         resps_list = first.generate_audio(text_list=[phns], proms_list=[proms], resp_lens=lens, seed=args.seed,
-                                          sample_steps=args.steps, known_list=known_list)
+                                          sample_steps=args.steps, known_list=known_list, temperature=args.temperature)
     else:
         nar = _load(args.nar_ckpt, args.device)
         if isinstance(first, DiscreteAR):       # the reference's own D3PM class: level 0 by diffusion, 350 frames
-            resp_list = [first.generate_audio([phns], [proms], seed=args.seed)[:350]]
+            resp_list = [first.generate_audio([phns], [proms], seed=args.seed, temperature=args.temperature)[:350]]
         else:
             resp_list = first(text_list=[phns], proms_list=[proms])
         resps_list = [r.unsqueeze(-1) for r in resp_list]
-        resps_list = nar(text_list=[phns], proms_list=[proms], resps_list=resps_list)
+        resps_list = nar(text_list=[phns], proms_list=[proms], resps_list=resps_list,
+                         sampling_temperature=args.nar_temperature, seed=args.seed)
     qnt.decode_to_file(resps=resps_list[0], path=args.out_path)
     print(args.out_path, "saved.")
 

@@ -56,6 +56,15 @@ PROTOTYPES = {
         [_p, _p, C.c_int, _p, C.c_int, _p, _p, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p, _u64,
          _p, _p],
         C.c_int),
+    "vb200_posterior_sample_from_logits_temp": (
+        [_p, _p, _p, C.c_int, _i64, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, C.c_int, C.c_int, _p, _u64, _p, _f, _p],
+        C.c_int),
+    "vb200_head_posterior_sample_temp": (
+        [_p, _p, C.c_int, _p, C.c_int, _p, _p, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p, _u64,
+         _p, _f, _p],
+        C.c_int),
+    "vb200_head_categorical_sample": (
+        [_p, _i64, _i32, _p, C.c_int, _p, C.c_int, _p, _p, _i32, _i32, _i32, _p, _p, _f, C.c_int, _u64, _p], C.c_int),
     "vb200_q_sample_philox": ([_p] * 5 + [_i32, _i32, _i32, C.c_int, _u64, _p], C.c_int),
     "vb200_head_fused": ([_i32, _i32, C.c_int], C.c_int),
     "vb200_head_ce_loss": ([_p, _p, C.c_int, _p, _p, _p, _i32, _i32, _i32, _i32, _p], C.c_int),
@@ -212,38 +221,41 @@ def q_sample_dense(x_out, x0, t_tok, mask, uniforms, log_qbar):
 
 
 def posterior_sample_from_logits(x_out, post_out, logits, ld_logits, x_t, row_utt, t_utt, utt, table,
-                                 n_rows, n_levels, K, transition, noise, uniforms=None, seed=0, known=None):
-    """``known``: int32 (n_rows, n_levels), -1 = draw as usual, k in [0, K) = the token's x0 is k (the ``_known``
-    entry point); None calls the plain one."""
-    if known is None:
-        _check(load().vb200_posterior_sample_from_logits(
-            ptr(x_out), ptr(post_out), ptr(logits), dtype_code(logits.dtype), ld_logits, ptr(x_t),
-            ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), n_rows, n_levels, K, table.shape[0], transition,
-            noise, ptr(uniforms), seed, stream()), "vb200_posterior_sample_from_logits")
-        return
-    _check(load().vb200_posterior_sample_from_logits_known(
+                                 n_rows, n_levels, K, transition, noise, uniforms=None, seed=0, known=None,
+                                 temperature=1.0):
+    """``known``: int32 (n_rows, n_levels) or None, -1 = draw as usual, k in [0, K) = the token's x0 is k.
+    ``temperature``: p̂(x0) = softmax(logits / temperature) (1.0: the unscaled step bit for bit)."""
+    _check(load().vb200_posterior_sample_from_logits_temp(
         ptr(x_out), ptr(post_out), ptr(logits), dtype_code(logits.dtype), ld_logits, ptr(x_t),
         ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), n_rows, n_levels, K, table.shape[0], transition,
-        noise, ptr(uniforms), seed, ptr(known), stream()), "vb200_posterior_sample_from_logits_known")
+        noise, ptr(uniforms), seed, ptr(known), temperature, stream()), "vb200_posterior_sample_from_logits_temp")
 
 
 def head_posterior_sample(x_out, logits, head_in, W, bias, x_t, row_utt, t_utt, utt, table, n_levels, K,
-                          transition, noise, uniforms=None, seed=0, known=None):
+                          transition, noise, uniforms=None, seed=0, known=None, temperature=1.0):
     """classifier + reverse step in one C call: one kernel (reverse step as the GEMM epilogue) when
     head_fused(), else GEMM into the caller's `logits` scratch (required then) + standalone kernel.
-    ``known`` as in posterior_sample_from_logits."""
+    ``known`` and ``temperature`` as in posterior_sample_from_logits."""
     n_rows, d = head_in.shape
     ldt = dtype_code(logits.dtype) if logits is not None else dtype_code(torch.float16)
-    if known is None:
-        _check(load().vb200_head_posterior_sample(
-            ptr(x_out), ptr(logits), ldt, ptr(head_in), act_code(head_in), ptr(W), ptr(bias), n_rows, d,
-            n_levels, K, ptr(x_t), ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), table.shape[0], transition,
-            noise, ptr(uniforms), seed, stream()), "vb200_head_posterior_sample")
-        return
-    _check(load().vb200_head_posterior_sample_known(
+    _check(load().vb200_head_posterior_sample_temp(
         ptr(x_out), ptr(logits), ldt, ptr(head_in), act_code(head_in), ptr(W), ptr(bias), n_rows, d,
         n_levels, K, ptr(x_t), ptr(row_utt), ptr(t_utt), ptr(utt), ptr(table), table.shape[0], transition,
-        noise, ptr(uniforms), seed, ptr(known), stream()), "vb200_head_posterior_sample_known")
+        noise, ptr(uniforms), seed, ptr(known), temperature, stream()), "vb200_head_posterior_sample_temp")
+
+
+def head_categorical_sample(x_out, col, logits, head_in, W, bias, row_utt, utt, temperature, noise=NOISE_PHILOX,
+                            seed=0):
+    """x_out[r, col] ~ softmax((head_in[r] W^T + bias) / temperature) for every row r of int32 x_out (n_rows, ld);
+    the other columns are not written.  One kernel when head_fused(d, K, noise), else GEMM into the caller's
+    ``logits`` scratch (n_rows, K) (required then) + one-warp-per-row draw.  Philox draws are keyed by (seed, global
+    utterance id from ``utt``, frame * ld + col)."""
+    n_rows, d = head_in.shape
+    K = W.shape[0]
+    ldt = dtype_code(logits.dtype) if logits is not None else dtype_code(torch.float16)
+    _check(load().vb200_head_categorical_sample(
+        ptr(x_out), x_out.shape[1], col, ptr(logits), ldt, ptr(head_in), act_code(head_in), ptr(W), ptr(bias),
+        n_rows, d, K, ptr(row_utt), ptr(utt), temperature, noise, seed, stream()), "vb200_head_categorical_sample")
 
 
 def q_sample_philox(x_out, x0, t_tok, mask, table, K, transition, seed=0):

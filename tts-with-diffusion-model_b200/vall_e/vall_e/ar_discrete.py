@@ -157,11 +157,13 @@ class AR(D3PMOps, nn.Module):
     # ------------------------------------------------------------------ reverse loop (:696-780)
     @torch.no_grad()
     def generate_audio(self, text_list, proms_list, resps_list=None, *, seed: int | None = None,
-                       greedy: bool = False, noise_fn=None) -> Tensor:
+                       greedy: bool = False, noise_fn=None, temperature: float = 1.0) -> Tensor:
         """x_T = 350 frames of the absorbing class in a 448 window, t = 99 .. 1, returns the (448,)
         level-0 codes like the reference.  Noise: ``torch.rand`` uniforms on the CPU generator as the
         reference (default), ``noise_fn(t) -> (1, 448, 1025)`` supplied uniforms, in-kernel Philox when
-        ``seed`` is given, or none (``greedy``)."""
+        ``seed`` is given, or none (``greedy``).  ``temperature``: p̂(x0) = softmax(logits / temperature) in every
+        reverse step (``D3PMOps.p_sample``); ValueError unless it is a finite number > 0."""
+        temperature = self._temperature(temperature)
         if len(text_list) != 1 or len(proms_list) != 1:
             raise ValueError("the reference's D3PM sampler handles one utterance per call (ar_discrete.py:699-712)")
         dev = self.final.weight.device
@@ -173,6 +175,6 @@ class AR(D3PMOps, nn.Module):
             t = torch.full((1,), step, dtype=torch.long, device=dev)
             logits = self.denoise_logits(x, t, cond1, cond2, mask)
             noise = noise_fn(step) if noise_fn is not None else None
-            x, _ = self.p_sample(logits, t, x, noise=noise, greedy=greedy, seed=seed)
+            x, _ = self.p_sample(logits, t, x, noise=noise, greedy=greedy, seed=seed, temperature=temperature)
             x = x.to(torch.int32)
         return x.squeeze().long()

@@ -12,6 +12,7 @@ Method names, argument order and tensor shapes follow the reference so parity te
 """
 from __future__ import annotations
 
+import math
 import numbers
 
 import torch
@@ -57,6 +58,14 @@ class D3PMOps:
             raise ValueError(f"sample_steps must be an integer in [1, {S - 1}] for a model with {S} timesteps, "
                              f"got {sample_steps!r}")
         return int(n)
+
+    @staticmethod
+    def _temperature(temperature) -> float:
+        """``temperature`` as a float, or ValueError for anything but a finite real number > 0 (bool refused)."""
+        ok = isinstance(temperature, numbers.Real) and not isinstance(temperature, bool)
+        if not ok or not math.isfinite(float(temperature)) or not float(temperature) > 0:
+            raise ValueError(f"temperature must be a finite number > 0, got {temperature!r}")
+        return float(temperature)
 
     def _sampling(self, device, n: int) -> tuple:
         """(schedule, its table, its int32 (S,) successor vector) of a reverse loop of n denoise steps."""
@@ -104,7 +113,7 @@ class D3PMOps:
 
     # ------------------------------------------------------------------ reverse step (row P)
     def _posterior(self, model_logits: Tensor, t: Tensor, x: Tensor, noise_mode: int, noise, want_post: bool,
-                   seed: int = 0, known: Tensor | None = None):
+                   seed: int = 0, known: Tensor | None = None, temperature: float = 1.0):
         B, W, K = model_logits.shape
         if K != self.num_classes:
             raise ValueError(f"logits have {K} classes, model has {self.num_classes}")
@@ -125,15 +134,20 @@ class D3PMOps:
         with torch.cuda.device(dev):
             L.posterior_sample_from_logits(out, post, logits, K, x_t, row_utt, t_utt, utt, self._table(dev),
                                            B * W, 1, K, _TRANSITIONS[self.transition], noise_mode, uni, seed,
-                                           known.to(dev) if known is not None else None)
+                                           known.to(dev) if known is not None else None, temperature)
         return out.view(B, W).long(), (post.view(B, W, K) if want_post else None)
 
-    def q_posterior_logits(self, x_start: Tensor, x_t: Tensor, t: Tensor, x_start_logits: bool = True) -> Tensor:
+    def q_posterior_logits(self, x_start: Tensor, x_t: Tensor, t: Tensor, x_start_logits: bool = True,
+                           temperature: float = 1.0) -> Tensor:
         """logits of q(x_{t-1} | x_t, p(x_0)) (ar_discrete.py:347-375), fp32 closed form.  ``x_start_logits=False``:
         x_start holds the ids of x0 (B, W) and this is q(x_{t-1} | x_t, x0) — the reference's ids branch, through
-        vb200_posterior_sample_from_logits_known with every token known (0 at t == 0, as the reference returns)."""
+        vb200_posterior_sample_from_logits_known with every token known (0 at t == 0, as the reference returns).
+        ``temperature`` (logits form): p(x_0) = softmax(x_start / temperature); t == 0 returns the raw logits."""
+        temperature = self._temperature(temperature)
         if x_start_logits:
-            return self._posterior(x_start, t, x_t, L.NOISE_GREEDY, None, want_post=True)[1]
+            return self._posterior(x_start, t, x_t, L.NOISE_GREEDY, None, want_post=True, temperature=temperature)[1]
+        if temperature != 1.0:
+            raise ValueError("temperature applies to the logits form only (x_start_logits=True)")
         B, W = x_start.shape
         K = self.num_classes
         known = x_start.to(torch.int32).contiguous().view(-1)
@@ -143,10 +157,13 @@ class D3PMOps:
         return self._posterior(placeholder, t, x_t, L.NOISE_GREEDY, None, want_post=True, known=known)[1]
 
     def p_sample(self, model_logits: Tensor, t: Tensor, x: Tensor, noise: Tensor | None = None,
-                 greedy: bool = False, seed: int | None = None):
+                 greedy: bool = False, seed: int | None = None, temperature: float = 1.0):
         """(sample (B, W) int64, softmax(model_logits)) like ar_discrete.py:401-420.  ``noise``:
         supplied uniforms (B, W, K); omitted -> torch.rand on the CPU generator as the reference,
-        unless ``seed`` is given (in-kernel Philox) or ``greedy``."""
+        unless ``seed`` is given (in-kernel Philox) or ``greedy``.  ``temperature``: the posterior is formed
+        from p̂(x0) = softmax(model_logits / temperature) (t == 0 still returns the arg max of the raw logits);
+        ValueError unless it is a finite number > 0."""
+        temperature = self._temperature(temperature)
         if greedy:
             mode, noise = L.NOISE_GREEDY, None
         elif noise is None and seed is not None:
@@ -155,7 +172,8 @@ class D3PMOps:
             mode = L.NOISE_UNIFORMS
             if noise is None:
                 noise = torch.rand(size=x.shape + (self.num_classes,)).to(x.device)
-        sample, _ = self._posterior(model_logits, t, x, mode, noise, want_post=False, seed=seed or 0)
+        sample, _ = self._posterior(model_logits, t, x, mode, noise, want_post=False, seed=seed or 0,
+                                    temperature=temperature)
         return sample, F.softmax(model_logits, dim=-1)
 
 
@@ -214,7 +232,7 @@ class Diffusion(D3PMOps, Base):
                        resp_lens: list[int] | None = None, seed: int = 0, greedy: bool = False,
                        uniforms_fn=None, gids=None, use_graph: bool = True, trace: list | None = None,
                        to_host: bool = False, as_bqt: bool = False, sample_steps: int | None = None,
-                       known_list: list[Tensor] | None = None):
+                       known_list: list[Tensor] | None = None, temperature: float = 1.0):
         """x_T -> x_0 for a batch of utterances; returns [LongTensor (t'', 8)].
 
         x_T is all ``mask_id`` for the absorbing transition (ar_discrete.py:699) and uniform random
@@ -234,8 +252,12 @@ class Diffusion(D3PMOps, Base):
         known levels).  Its lengths define ``resp_lens``.  Known tokens start from the same x_T as the others and
         draw every step from the exact posterior q(x_s | x_t, x0 = k); the returned codes equal the given ones at
         every known position (DESIGN.md §5).
+        ``temperature`` τ: every reverse step draws from the posterior on p̂(x0) = softmax(logits / τ); τ < 1
+        sharpens p̂(x0), τ = 1 (default) is the unscaled loop bit for bit.  Known tokens do not read their logits and
+        are unaffected.  ValueError unless τ is a finite number > 0 (DESIGN.md §5).
         """
         n_steps = self._sample_steps(sample_steps)
+        temperature = self._temperature(temperature)
         known = None
         if known_list is not None:      # checked before the device is touched, like sample_steps
             known, resp_lens = self._known(known_list, resp_lens, resps_list, len(text_list))
@@ -268,7 +290,7 @@ class Diffusion(D3PMOps, Base):
         noise = L.NOISE_GREEDY if greedy else (L.NOISE_UNIFORMS if uniforms_fn is not None else L.NOISE_PHILOX)
         ses.run(table, self.timesteps, _TRANSITIONS[self.transition], noise=noise, seed=seed,
                 uniforms_fn=uniforms_fn, use_graph=use_graph, n_levels=self.n_levels, trace=trace,
-                schedule=schedule, next_t=next_t, known=known)
+                schedule=schedule, next_t=next_t, known=known, temperature=temperature)
         if as_bqt:        # one (B, 8, T_max) int64 tensor in the EnCodec decoder's layout + the frame counts
             bqt = torch.empty(lay.B, self.n_levels, max(lay.t_resp), dtype=torch.int64, device=dev)
             with torch.cuda.device(dev):
